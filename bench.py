@@ -9,6 +9,7 @@ post-process + pseudo-label filter -> List[Instances] pseudo-labels, followed by
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [...]                         # the reference's CPU path (oracle) on the host cores
+    python bench.py [...] --dump-outputs DIR                       # + the last timed step's outputs as DIR/<name>.npy
 
 Under torchrun (N > 1) every rank owns a teacher replica and its own 8 images (no data-path collective: weak scaling);
 timing is barrier + synchronize on both sides, CUDA events, max over ranks; rank 0 prints ONE JSON line.
@@ -68,7 +69,16 @@ def parse_args():
                     help="bracket the timed region with cudaProfilerStart/Stop (for `ncu --profile-from-start off`); "
                          "numbers printed under a profiler are not bench values")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="wall-clock budget of the reference arm")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (RPN proposals, detections, pseudo-labels, "
+                         "a seeded sample of the EMA-updated teacher state) as DIR/<name>.npy, float32, so that two builds can be "
+                         "compared output for output (the inputs are seeded: the same arguments give the same inputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return args
 
 
 def peaks():
@@ -341,6 +351,54 @@ def flip_rate_sample(dev, seeds: int = 12):
         return {"error": repr(e)[:300]}
 
 
+# What one step returns (step_resident): per image, the RPN proposals, the Fast R-CNN detections and the pseudo-labels
+DUMP_FIELDS = (("rpn", ("proposal_boxes", "objectness_logits")),
+               ("detections", ("pred_boxes", "scores", "pred_classes")),
+               ("pseudo_labels", ("gt_boxes", "gt_classes", "scores")))
+DUMP_STATE_SAMPLE = 4096          # elements drawn from each floating-point tensor of the teacher state
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, out, teacher, max_rows):
+    """Writes the results ``out`` of the last timed step as float32 .npy files under ``out_dir``: every field of DUMP_FIELDS
+    as one (images, max_rows[list], ...) array (``<list>_<field>.npy``) whose rows past an image's count are zero, the rows of
+    each image (``<list>_per_image.npy``), and ``teacher_state_sample.npy``, a fixed, seeded sample of every floating-point
+    tensor of the teacher's state_dict (in state_dict order) after the step's EMA and train-mode BatchNorm running-statistic
+    updates.  The shapes follow from the configuration alone, so every file exists and two builds line up image by image
+    even where their counts differ (the random-init teacher of the benchmark scores no detection above the pseudo-label
+    threshold: its pseudo-label fields are all padding)."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for (name, fields), insts in zip(DUMP_FIELDS, out):
+        counts = [len(p) for p in insts]
+        if max(counts) > max_rows[name]:
+            raise RuntimeError(f"--dump-outputs: {name} has {max(counts)} rows in an image, more than {max_rows[name]}")
+        arrays[f"{name}_per_image"] = torch.tensor(counts, dtype=torch.float32)
+        for f in fields:
+            vals = [getattr(v, "tensor", v).float() for v in (p.get(f) for p in insts)]
+            padded = vals[0].new_zeros((len(vals), max_rows[name]) + vals[0].shape[1:])
+            for i, v in enumerate(vals):
+                padded[i, :len(v)] = v
+            arrays[f"{name}_{f}"] = padded
+    g = torch.Generator().manual_seed(0)
+    sample = []
+    for v in teacher.state_dict().values():
+        if v.is_floating_point():
+            flat = v.detach().reshape(-1)
+            n = flat.numel()
+            idx = torch.randint(n, (DUMP_STATE_SAMPLE,), generator=g) if n > DUMP_STATE_SAMPLE else torch.arange(n)
+            sample.append(flat[idx.to(flat.device)].float())
+    arrays["teacher_state_sample"] = torch.cat(sample)
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ B200 arm
 def run_b200(args):
     import torch
@@ -463,6 +521,9 @@ def run_b200(args):
     if args.profiler_range:
         torch.cuda.profiler.stop()
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        # before the other records below step the teacher further; the teacher runs in train() mode: the TRAIN proposal budget
+        dump_outputs(args.dump_outputs, out, teacher, {"rpn": cfg.MODEL.RPN.POST_NMS_TOPK_TRAIN, "detections": T, "pseudo_labels": T})
     for i in range(3):
         step_e2e(i)
     ms_e2e, _, _, _ = timed(step_e2e, args.steps)

@@ -1,7 +1,7 @@
 """Writes tests/golden/ref_exec.npz: inputs and outputs of the REFERENCE'S OWN functions, executed on the CPU from the sources
-under /root/reference (tests/ref_exec.py: nothing is copied, the code that runs is the reference's text).
+under $SFOD_REFERENCE_ROOT (tests/ref_exec.py: nothing is copied, the code that runs is the reference's text).
 
-    python tests/golden/make_golden_ref.py        # in the build container, where /root/reference is mounted
+    SFOD_REFERENCE_ROOT=<checkout of the original project> python tests/golden/make_golden_ref.py
 
 Functions executed (reference file:line):
   daod/modeling/roi_heads/fast_rcnn.py:88-142            fast_rcnn_inference_single_image_with_mcd   -> frcnn_*_out_*
@@ -67,7 +67,9 @@ def main():
                 out[f"frcnn_{i}_pl_{k}"] = pl[k].numpy()
                 out[f"frcnn_{i}_adaptive_{k}"] = ad[k].numpy()
             conv = R.fast_rcnn_inference_single_image_new(b.clone(), s.clone(), sz)
-            for k in ("pred_boxes", "scores", "pred_classes", "kept_rows"):
+            # its scores are s[kept_rows, pred_classes] bit for bit (a gather, no NMS): not stored, which keeps the file under 1 MB
+            assert torch.equal(conv["scores"], s[conv["kept_rows"], conv["pred_classes"]])
+            for k in ("pred_boxes", "pred_classes", "kept_rows"):
                 out[f"frcnn_{i}_conv_{k}"] = conv[k].numpy()
         reserve = tr.count_label_prediction(dets)
         out["reserve_count"] = reserve.numpy()

@@ -5,13 +5,13 @@ state the hot path's semantics are plain torch once three names resolve: ``Boxes
 ``sfod_b200.d2shim``, a detectron2 namespace backed by this package's structures), ``batched_nms`` (detectron2 0.6
 ``layers/nms.py``: ``torchvision.ops.boxes.batched_nms(boxes.float(), scores, idxs, iou_threshold)`` -- bound here to the
 installed torchvision CPU kernel) and ``comm.get_world_size``.  Module-level sources are imported from where they lie under
-/root/reference; trainer METHODS live in modules whose imports cannot be satisfied (DefaultTrainer, checkpointing, data
+$SFOD_REFERENCE_ROOT; trainer METHODS live in modules whose imports cannot be satisfied (DefaultTrainer, checkpointing, data
 loaders), so their ``def`` nodes are cut out of the parsed file and compiled in a small namespace -- the code that runs is the
 reference's text, byte for byte, and nothing is copied into this repository.  ``.cuda()`` calls inside those functions are
 neutralised (identity) for the duration of a call so that the CPU is the device.
 
 Used by tests/test_oracle_vs_reference_cpu.py (oracle/d2_cpu.py == reference, live) and tests/golden/make_golden_ref.py (writes
-tests/golden/ref_exec.npz, the fixture that travels to the GPU box where /root/reference does not exist).
+tests/golden/ref_exec.npz, the fixture that stands in for the reference wherever its sources are absent).
 """
 from __future__ import annotations
 
@@ -30,7 +30,8 @@ import torch
 import torchvision
 from torch import nn
 
-REF_ROOT = "/root/reference"
+# A checkout of the original project (the directory holding daod/); the tests that execute it skip without one.
+REF_ROOT = os.environ.get("SFOD_REFERENCE_ROOT", "")
 TRAINER = os.path.join(REF_ROOT, "daod/engine/trainers/source_free_adaptive_teacher.py")
 TRAINER_AT = os.path.join(REF_ROOT, "daod/engine/trainers/adaptive_teacher.py")
 BASE = os.path.join(REF_ROOT, "daod/engine/trainers/base.py")
@@ -38,7 +39,7 @@ ADAPTIVE = os.path.join(REF_ROOT, "daod/modeling/adaptive_thresh/adaptive_confid
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REF_ROOT, "daod"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "daod"))
 
 
 def d2_batched_nms(boxes, scores, idxs, iou_threshold):
@@ -87,7 +88,7 @@ def _compile_functions(path: str, names, namespace: dict):
 
 
 class Reference:
-    """Handles to the reference's functions, live from /root/reference.  Use as a context manager (installs / removes the shim)."""
+    """Handles to the reference's functions, live from REF_ROOT.  Use as a context manager (installs / removes the shim)."""
 
     def __enter__(self):
         import sfod_b200  # noqa: F401
