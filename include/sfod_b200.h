@@ -46,6 +46,7 @@ enum sfod_status {
 enum sfod_layout { SFOD_NCHW = 0, SFOD_NHWC = 1 };
 enum sfod_dtype { SFOD_F32 = 0, SFOD_I64 = 1, SFOD_U8 = 2 };
 
+/* Changes whenever an entry point keeps its name but changes its arguments; a binding refuses a library of another version. */
 int sfod_abi_version(void);
 /* sizeof() of the parameter structs as this library was compiled (which: 0 sfod_ema_tensor, 1 sfod_rpn_params,
  * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params; 0 for anything else) -- lets a foreign
@@ -102,9 +103,8 @@ int sfod_roi_pool_fwd(const float *input, const float *rois, int N, int C, int H
                       float spatial_scale, float *output, int32_t *argmax, sfod_stream_t stream);
 int sfod_roi_pool_bwd(const float *grad_out, const float *rois, const int32_t *argmax, int N, int C, int H, int W,
                       int R, int PH, int PW, float *grad_in, sfod_stream_t stream);
-/* layout helpers used by the wrappers (tiled shared-memory transposes) */
+/* layout helper used by the wrappers (tiled shared-memory transpose) */
 int sfod_nchw_to_nhwc(const float *src, float *dst, int N, int C, int HW, sfod_stream_t stream);
-int sfod_nhwc_to_nchw(const float *src, float *dst, int N, int C, int HW, sfod_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * NMS with torchvision semantics.  Replaces torchvision.ops.nms / batched_nms as reached
@@ -276,39 +276,38 @@ int sfod_subsample_labels(const int64_t *labels, const int32_t *offsets, int num
  * (daod/engine/trainers/base.py:274-299, after reset_bn_stats :318-323) and by the teacher
  * forward under no_grad (source_free_adaptive_teacher.py:385-390).
  * Phase 1 (sfod_bn_partial_stats): per-channel (sum x, sum x^2) over (N,H,W) accumulated
- *   in fp64 into stats_dev (C,2) doubles (zeroed by the call) -- the tensor a multi-GPU
- *   caller all-reduces (together with the element count) before phase 2.
- * Phase 2 (sfod_bn_finalize_apply): mean, biased var (fp64), running stats
- *   r = (1-m) r + m stat with the unbiased variance n/(n-1), num_batches_tracked += 1,
- *   y = (x-mean)*invstd*weight+bias (optionally fused ReLU); y may alias x.
- * stats_dev must hold sfod_bn_stats_bytes(C) bytes: the (C,2) totals, then scratch of the
+ *   in fp64 into stats_dev (C,2) doubles, and the element count N*H*W into stats_dev[2C]
+ *   (zeroed and written by the call).  These 2C+1 doubles are the payload a multi-GPU caller
+ *   sums over the ranks before phase 2: with an all-reduce of its own (NCCL), or with the
+ *   peer-memory exchange below.
+ * Phase 2 (sfod_bn_finalize_apply): mean, biased var (fp64) from the totals and the count,
+ *   both read on the device (a multi-GPU AdaBN forward needs no host read between its two
+ *   phases: reference daod/engine/trainers/base.py:270-337 on several ranks; SURVEY.md 8e
+ *   collective 2), running stats r = (1-m) r + m stat with the unbiased variance n/(n-1),
+ *   num_batches_tracked += 1, y = (x-mean)*invstd*weight+bias (optionally fused ReLU); y may
+ *   alias x.  x or y NULL: statistics and running statistics only.
+ * comm (both phases; NULL = the statistics in stats_dev are used as they are): the peer-memory exchange below.
+ * stats_dev must hold sfod_bn_stats_bytes(C) bytes: the 2C+1 payload, then scratch of the
  * library (scale/shift of phase 2, replicated partial totals of the channels-last pass). */
 size_t sfod_bn_stats_bytes(int C);
+typedef struct sfod_p2p_comm sfod_p2p_comm_t; /* defined with the peer-memory exchange below */
 /* pre_bias (C floats, may be NULL): a per-channel bias added to x before everything else -- the bias of the
  * convolution that feeds the BatchNorm (reference daod/modeling/meta_arch/vgg.py:17-19: Conv2d(bias=True) -> BatchNorm2d),
  * so that the convolution can run bias-free and its separate elementwise pass over the activation disappears.
  * Statistics, running statistics and output are those of fl(x + pre_bias[c]), bit-identical to adding the bias first. */
 int sfod_bn_partial_stats(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                          sfod_stream_t stream);
-/* fuse_maxpool2 != 0: y is the (N,C,H/2,W/2) result of MaxPool2d(kernel_size=2, stride=2) applied to the normalised
+                          const sfod_p2p_comm_t *comm, sfod_stream_t stream);
+/* residual (same shape and layout as x, may be NULL; SFOD_ERR_ALIGNMENT unless it has x's 16-byte phase):
+ * y = [relu](fl(bn(x)) + residual) -- the tail of a detectron2 BottleneckBlock (conv3+norm, `out += shortcut`, `relu_`),
+ * which the R101-C4 configs of the reference (configs/r101_c4_cs_foggy_adaptive_teacher_source_free.yaml:5-7,
+ * RESNETS.NORM "BN") execute as three elementwise passes.
+ * fuse_maxpool2 != 0: y is the (N,C,H/2,W/2) result of MaxPool2d(kernel_size=2, stride=2) applied to the normalised
  * (+ReLU) activation (vgg.py:15), written directly (x is read once, the full-resolution activation is never stored);
- * y must not alias x in that mode. */
-int sfod_bn_finalize_apply(const float *x, const float *pre_bias, float *y, int layout, int N, int C, int H, int W,
-                           const double *stats_dev, double total_count, const float *weight, const float *bias,
-                           float *running_mean, float *running_var, int64_t *num_batches_tracked, double momentum,
-                           double eps, int fuse_relu, int fuse_maxpool2, float *save_mean, float *save_invstd,
-                           sfod_stream_t stream);
-/* v2 adds (i) `residual` (same shape and layout as x, may be NULL): y = [relu](fl(bn(x)) + residual) -- the tail of a
- * detectron2 BottleneckBlock (conv3+norm, `out += shortcut`, `relu_`), which the R101-C4 configs of the reference
- * (configs/r101_c4_cs_foggy_adaptive_teacher_source_free.yaml:5-7, RESNETS.NORM "BN") execute as three elementwise passes;
- * (ii) `count_on_device` != 0: the element count is read from stats_dev[2*C] on the device (phase 1 writes the local count
- * there, an all-reduce of the first 2C+1 doubles makes it global), so a multi-GPU AdaBN forward needs no host read between
- * its two phases (reference daod/engine/trainers/base.py:270-337 on several ranks; SURVEY.md 8e collective 2). */
-int sfod_bn_finalize_apply_v2(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N, int C,
-                              int H, int W, const double *stats_dev, double total_count, int count_on_device,
-                              const float *weight, const float *bias, float *running_mean, float *running_var,
-                              int64_t *num_batches_tracked, double momentum, double eps, int fuse_relu, int fuse_maxpool2,
-                              float *save_mean, float *save_invstd, sfod_stream_t stream);
+ * y must not alias x and residual must be NULL in that mode. */
+int sfod_bn_finalize_apply(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N, int C,
+                           int H, int W, double *stats_dev, const sfod_p2p_comm_t *comm, const float *weight, const float *bias,
+                           float *running_mean, float *running_var, int64_t *num_batches_tracked, double momentum, double eps,
+                           int fuse_relu, int fuse_maxpool2, sfod_stream_t stream);
 /* Single-launch variant of phase 1 + phase 2 for NCHW activations that (mostly) fit the 126 MB L2 (late VGG layers, res3 / res4
  * of R101-C4): a cooperative persistent kernel computes the statistics, crosses one grid barrier and normalises the chunks it has
  * just read in reverse order, so the second read of x comes from L2 (~8 instead of 12 B/element of HBM traffic, 1 launch instead
@@ -333,8 +332,15 @@ int sfod_bn_frozen_apply(const float *x, const float *residual, float *y, int la
  * test_refinement (reference daod/engine/trainers/base.py:270-337) or the teacher forward
  * (source_free_adaptive_teacher.py:385-390) runs data-parallel.  Instead of a collective launch per layer (NCCL
  * all-reduce of 2C+1 doubles: the baseline, see simple-sfod_b200/engine/adabn_dist.py) the exchange is fused into phase 2:
- * one kernel stores the local payload into every peer's inbox with P2P stores, raises a flag per peer, waits for the
- * peers' flags, adds the payloads in rank order (bit-identical totals on every rank) and computes the coefficients.
+ * sfod_bn_finalize_apply with comm != NULL runs one kernel that stores the local payload into every peer's inbox with P2P
+ * stores (every element tagged with the exchange's epoch), polls for the peers' elements, adds the payloads in rank order
+ * (bit-identical totals on every rank), leaves these totals of the concatenated batch in stats_dev and computes the
+ * coefficients.  sfod_bn_partial_stats with comm != NULL computes the same statistics; in addition the CTA of the statistics
+ * kernel that finishes last delivers the payload to the peers' inboxes (NCHW layers covered by one launch; otherwise phase 2
+ * delivers it), so the NVLink transfer overlaps the launch gap between the two phases.  It must then be followed by
+ * sfod_bn_finalize_apply on the same stream, comm and stats_dev.  With comm != NULL both calls return SFOD_ERR_INVALID_ARG
+ * unless 1 <= world <= SFOD_P2P_MAX_RANKS, 0 <= rank < world and every inbox[r] is set, and SFOD_ERR_UNSUPPORTED for
+ * C > sfod_p2p_max_channels().
  *
  * An inbox is sfod_p2p_inbox_bytes() of device memory allocated by sfod_p2p_alloc (cudaMalloc + zero fill), which also
  * returns its 64-byte CUDA IPC handle; the caller ships the handle to the other processes of the node (any host channel:
@@ -344,10 +350,10 @@ int sfod_bn_frozen_apply(const float *x, const float *residual, float *y, int la
  * results of a timed-out exchange are invalid) -- the GPU is never left spinning. */
 #define SFOD_P2P_MAX_RANKS 8
 #define SFOD_P2P_HANDLE_BYTES 64
-typedef struct sfod_p2p_comm {
+struct sfod_p2p_comm {
   int32_t rank, world;                 /* world <= SFOD_P2P_MAX_RANKS */
   void *inbox[SFOD_P2P_MAX_RANKS];     /* inbox[r]: rank r's inbox as mapped into THIS process (inbox[rank] = own allocation) */
-} sfod_p2p_comm_t;
+};
 size_t sfod_p2p_inbox_bytes(void);
 int sfod_p2p_max_channels(void);       /* largest C one exchange carries (2051: covers the 2048-channel res5 of the reference backbones) */
 int sfod_p2p_alloc(void **inbox, unsigned char *handle /* SFOD_P2P_HANDLE_BYTES, may be NULL */);
@@ -356,19 +362,6 @@ int sfod_p2p_close(void *peer_inbox);
 int sfod_p2p_free(void *inbox);
 /* Synchronous read of the own inbox header: exchanges completed, exchanges abandoned on a timeout. */
 int sfod_p2p_status(const sfod_p2p_comm_t *comm, uint64_t *exchanges, uint32_t *timeouts);
-/* sfod_bn_partial_stats for a rank of `comm`: same result in stats_dev; in addition the CTA of the statistics kernel that
- * finishes last delivers the payload to the peers' inboxes (NCHW layers covered by one launch; otherwise phase 2 delivers it),
- * so the NVLink transfer overlaps the launch gap between the two phases.  Must be followed by
- * sfod_bn_exchange_finalize_apply on the same stream, comm and stats_dev. */
-int sfod_bn_partial_stats_p2p(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                              const sfod_p2p_comm_t *comm, sfod_stream_t stream);
-/* sfod_bn_finalize_apply_v2 with the cross-rank exchange in front of it: stats_dev holds this rank's phase-1 result
- * ((C,2) totals and the local element count at [2C]) on entry and the totals of the concatenated batch on return. */
-int sfod_bn_exchange_finalize_apply(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N,
-                                    int C, int H, int W, double *stats_dev, const sfod_p2p_comm_t *comm, const float *weight,
-                                    const float *bias, float *running_mean, float *running_var, int64_t *num_batches_tracked,
-                                    double momentum, double eps, int fuse_relu, int fuse_maxpool2, float *save_mean,
-                                    float *save_invstd, sfod_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------------------
  * Strong augmentation of the student's input on the device (SURVEY.md 8f rank 3).  Replaces the PIL / torchvision CPU

@@ -54,6 +54,11 @@ class P2PComm(C.Structure):
     _fields_ = [("rank", C.c_int32), ("world", C.c_int32), ("inbox", C.c_void_p * P2P_MAX_RANKS)]
 
 
+# sfod_abi_version() of the library this binding is written for, and the struct mirrors in the order of sfod_abi_sizeof(which)
+ABI_VERSION = 2
+ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams)
+
+
 # name -> (restype, argtypes); every symbol include/sfod_b200.h declares
 SIGNATURES = {
     "sfod_abi_version": (C.c_int, []),
@@ -73,7 +78,6 @@ SIGNATURES = {
     "sfod_roi_pool_fwd": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 7 + [C.c_float, c_ptr, c_ptr, c_ptr]),
     "sfod_roi_pool_bwd": (C.c_int, [c_ptr, c_ptr, c_ptr] + [C.c_int] * 7 + [c_ptr, c_ptr]),
     "sfod_nchw_to_nhwc": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
-    "sfod_nhwc_to_nchw": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
     "sfod_nms_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "sfod_nms": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int64, C.c_double, C.c_int64, c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "sfod_rpn_select_workspace_bytes": (C.c_size_t, [C.POINTER(RpnParams)]),
@@ -97,9 +101,9 @@ SIGNATURES = {
     "sfod_random_erase": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_uint64, c_ptr]),
     "sfod_subsample_labels": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_uint64, c_ptr, c_ptr, c_ptr]),
     "sfod_bn_stats_bytes": (C.c_size_t, [C.c_int]),
-    "sfod_bn_partial_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, c_ptr]),
-    "sfod_bn_finalize_apply": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.c_double, c_ptr, c_ptr,
-                                         c_ptr, c_ptr, c_ptr, C.c_double, C.c_double, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr]),
+    "sfod_bn_partial_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, C.POINTER(P2PComm), c_ptr]),
+    "sfod_bn_finalize_apply": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.POINTER(P2PComm),
+                                         c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_double, C.c_double, C.c_int, C.c_int, c_ptr]),
     "sfod_bn_train_fused": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                       C.c_double, C.c_double, C.c_int, c_ptr]),
     "sfod_bn_frozen_scratch_bytes": (C.c_size_t, [C.c_int]),
@@ -112,12 +116,6 @@ SIGNATURES = {
     "sfod_p2p_close": (C.c_int, [c_ptr]),
     "sfod_p2p_free": (C.c_int, [c_ptr]),
     "sfod_p2p_status": (C.c_int, [C.POINTER(P2PComm), C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
-    "sfod_bn_partial_stats_p2p": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, C.POINTER(P2PComm), c_ptr]),
-    "sfod_bn_exchange_finalize_apply": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr,
-                                                  C.POINTER(P2PComm), c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_double, C.c_double, C.c_int,
-                                                  C.c_int, c_ptr, c_ptr, c_ptr]),
-    "sfod_bn_finalize_apply_v2": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.c_double, C.c_int,
-                                            c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_double, C.c_double, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr]),
 }
 
 
@@ -145,8 +143,21 @@ def lib() -> C.CDLL:
             fn = getattr(handle, name)  # AttributeError if the symbol is not exported
             fn.restype = res
             fn.argtypes = args
+        _check_abi(handle)
         _lib = handle
     return _lib
+
+
+def _check_abi(handle: C.CDLL) -> None:
+    """Refuse a library built from another revision of the header: ctypes would hand it argument lists it does not expect."""
+    version = handle.sfod_abi_version()
+    if version != ABI_VERSION:
+        raise SfodLibraryError(f"{LIB_PATH} has ABI version {version}, this binding expects {ABI_VERSION}: rebuild it "
+                               "(`python simple-sfod_b200/build.py --force`)")
+    for which, mirror in enumerate(ABI_STRUCTS):
+        size = handle.sfod_abi_sizeof(which)
+        if size != C.sizeof(mirror):
+            raise SfodLibraryError(f"{LIB_PATH}: struct {which} has {size} bytes, its ctypes mirror {mirror.__name__} {C.sizeof(mirror)}")
 
 
 def check(status: int, what: str = "") -> None:

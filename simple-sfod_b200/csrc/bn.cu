@@ -229,15 +229,12 @@ __global__ void __launch_bounds__(kThreads) bn_stats_nhwc_scalar_kernel(const fl
 __device__ __forceinline__ void bn_finalize_channel(int c, double sum, double sumsq, double n, const float *__restrict__ weight,
                                                     const float *__restrict__ bias, float *__restrict__ running_mean,
                                                     float *__restrict__ running_var, double momentum, double eps,
-                                                    float *__restrict__ save_mean, float *__restrict__ save_invstd,
                                                     float *__restrict__ scale, float *__restrict__ shift) {
   const double mean = sum / n;
   double var = sumsq / n - mean * mean;
   if (var < 0.0) var = 0.0;
   const double invstd = 1.0 / sqrt(var + eps);
   const float mean_f = (float)mean;
-  if (save_mean) save_mean[c] = mean_f;
-  if (save_invstd) save_invstd[c] = (float)invstd;
   if (running_mean) running_mean[c] = (float)(momentum * (double)mean_f + (1.0 - momentum) * (double)running_mean[c]);
   if (running_var) {
     const double unbiased = n > 1.0 ? var * n / (n - 1.0) : var;
@@ -249,17 +246,15 @@ __device__ __forceinline__ void bn_finalize_channel(int c, double sum, double su
 }
 
 // One thread per channel.
-__global__ void bn_finalize_kernel(const double *__restrict__ stats, int C, double n_host, int count_on_device, const float *__restrict__ weight,
+__global__ void bn_finalize_kernel(const double *__restrict__ stats, int C, const float *__restrict__ weight,
                                    const float *__restrict__ bias, float *__restrict__ running_mean,
                                    float *__restrict__ running_var, long long *__restrict__ nbt, double momentum, double eps,
-                                   float *__restrict__ save_mean, float *__restrict__ save_invstd, float *__restrict__ scale,
-                                   float *__restrict__ shift) {
+                                   float *__restrict__ scale, float *__restrict__ shift) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c == 0 && nbt) *nbt += 1;
   if (c >= C) return;
-  const double n = count_on_device ? stats[2 * C] : n_host;   // all-reduced element count: no host read between the phases
-  bn_finalize_channel(c, stats[2 * c], stats[2 * c + 1], n, weight, bias, running_mean, running_var, momentum, eps, save_mean,
-                      save_invstd, scale, shift);
+  const double n = stats[2 * C];   // element count left by phase 1 (and summed over the ranks by an all-reduce): no host read between the phases
+  bn_finalize_channel(c, stats[2 * c], stats[2 * c + 1], n, weight, bias, running_mean, running_var, momentum, eps, scale, shift);
 }
 
 template <bool kRelu>
@@ -557,23 +552,10 @@ static bool p2p_comm_ok(const sfod_p2p_comm_t *comm) {
   return true;
 }
 
-static int bn_partial_stats_impl(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                                 const sfod_p2p_comm_t *comm, sfod_stream_t stream);
-
 SFOD_API int sfod_bn_partial_stats(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                                   sfod_stream_t stream) {
-  return bn_partial_stats_impl(x, pre_bias, layout, N, C, HW, stats_dev, nullptr, stream);
-}
-
-SFOD_API int sfod_bn_partial_stats_p2p(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                                       const sfod_p2p_comm_t *comm, sfod_stream_t stream) {
-  if (!p2p_comm_ok(comm)) return SFOD_ERR_INVALID_ARG;
-  if (2 * C + 1 > kP2PMaxPayload) return SFOD_ERR_UNSUPPORTED;
-  return bn_partial_stats_impl(x, pre_bias, layout, N, C, HW, stats_dev, comm, stream);
-}
-
-static int bn_partial_stats_impl(const float *x, const float *pre_bias, int layout, int N, int C, int64_t HW, double *stats_dev,
-                                 const sfod_p2p_comm_t *comm, sfod_stream_t stream) {
+                                   const sfod_p2p_comm_t *comm, sfod_stream_t stream) {
+  if (comm && !p2p_comm_ok(comm)) return SFOD_ERR_INVALID_ARG;
+  if (comm && 2 * C + 1 > kP2PMaxPayload) return SFOD_ERR_UNSUPPORTED;
   if (!x || !stats_dev || N <= 0 || C <= 0 || HW <= 0) return SFOD_ERR_INVALID_ARG;
   if (layout != SFOD_NCHW && layout != SFOD_NHWC) return SFOD_ERR_INVALID_ARG;
   cudaStream_t st = sfod_cu(stream);
@@ -696,32 +678,7 @@ int launch_bn_apply(const float *x, const float *pre_bias, const float *residual
   SFOD_LAUNCH_CHECK();
   return SFOD_OK;
 }
-}  // namespace
 
-// stats_dev layout: [0, 2C) (sum x, sum x^2); [2C] element count of this rank (written by phase 1; with [0, 2C) it forms the
-// 2C+1 all-reduce payload); [2C + 2, ...) float scale / shift scratch of phase 2; [4C, ...) replica totals of the NHWC pass.
-SFOD_API int sfod_bn_finalize_apply_v2(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N, int C,
-                                       int H, int W, const double *stats_dev, double total_count, int count_on_device,
-                                       const float *weight, const float *bias, float *running_mean, float *running_var,
-                                       int64_t *num_batches_tracked, double momentum, double eps, int fuse_relu, int fuse_maxpool2,
-                                       float *save_mean, float *save_invstd, sfod_stream_t stream) {
-  if (!stats_dev || N <= 0 || C <= 0 || H <= 0 || W <= 0 || (!count_on_device && total_count <= 0)) return SFOD_ERR_INVALID_ARG;
-  if (layout != SFOD_NCHW && layout != SFOD_NHWC) return SFOD_ERR_INVALID_ARG;
-  if (residual && fuse_maxpool2) return SFOD_ERR_INVALID_ARG;
-  if (residual && x && ((reinterpret_cast<uintptr_t>(residual) ^ reinterpret_cast<uintptr_t>(x)) & 15u)) return SFOD_ERR_ALIGNMENT;
-  cudaStream_t st = sfod_cu(stream);
-  const long long HW = (long long)H * W;
-  float *scale = reinterpret_cast<float *>(const_cast<double *>(stats_dev) + 2 * (size_t)C + 2);
-  float *shift = scale + sfod_align_up((size_t)C, 4);
-  bn_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(stats_dev, C, total_count, count_on_device, weight, bias, running_mean, running_var,
-                                                      reinterpret_cast<long long *>(num_batches_tracked), momentum, eps,
-                                                      save_mean, save_invstd, scale, shift);
-  SFOD_LAUNCH_CHECK();
-  if (!x || !y) return SFOD_OK;  // statistics-only mode (AdaBN does not need the normalised output of the last layer)
-  return launch_bn_apply(x, pre_bias, residual, y, layout, N, C, H, W, scale, shift, fuse_relu, fuse_maxpool2, st);
-}
-
-namespace {
 // FrozenBatchNorm2d / eval-mode BatchNorm coefficients: y = x * scale + shift with scale = w / sqrt(running_var + eps),
 // shift = b - running_mean * scale (detectron2 layers/batch_norm.py FrozenBatchNorm2d.forward, fp32 like the reference).
 __global__ void bn_frozen_coeffs_kernel(int C, const float *__restrict__ weight, const float *__restrict__ bias,
@@ -735,15 +692,6 @@ __global__ void bn_frozen_coeffs_kernel(int C, const float *__restrict__ weight,
   shift[c] = __fsub_rn(b, __fmul_rn(running_mean[c], sc));
 }
 }  // namespace
-
-SFOD_API int sfod_bn_finalize_apply(const float *x, const float *pre_bias, float *y, int layout, int N, int C, int H, int W,
-                                    const double *stats_dev, double total_count, const float *weight, const float *bias,
-                                    float *running_mean, float *running_var, int64_t *num_batches_tracked, double momentum,
-                                    double eps, int fuse_relu, int fuse_maxpool2, float *save_mean, float *save_invstd,
-                                    sfod_stream_t stream) {
-  return sfod_bn_finalize_apply_v2(x, pre_bias, nullptr, y, layout, N, C, H, W, stats_dev, total_count, 0, weight, bias, running_mean,
-                                   running_var, num_batches_tracked, momentum, eps, fuse_relu, fuse_maxpool2, save_mean, save_invstd, stream);
-}
 
 SFOD_API size_t sfod_bn_frozen_scratch_bytes(int C) { return C > 0 ? sfod_align_up(2 * sfod_align_up((size_t)C, 4) * sizeof(float), 256) : 256; }
 
@@ -824,7 +772,6 @@ __global__ void __launch_bounds__(kP2PThreads) bn_exchange_finalize_kernel(doubl
                                                                             const float *__restrict__ weight, const float *__restrict__ bias,
                                                                             float *__restrict__ running_mean, float *__restrict__ running_var,
                                                                             long long *__restrict__ nbt, double momentum, double eps,
-                                                                            float *__restrict__ save_mean, float *__restrict__ save_invstd,
                                                                             float *__restrict__ scale, float *__restrict__ shift) {
   __shared__ double tot[kP2PMaxPayload];
   __shared__ int s_timeout;
@@ -860,8 +807,7 @@ __global__ void __launch_bounds__(kP2PThreads) bn_exchange_finalize_kernel(doubl
   for (int i = threadIdx.x; i < n; i += blockDim.x) stats[i] = tot[i];   // the totals of the concatenated batch, as the NCCL path leaves them
   const double cnt = tot[2 * C];
   for (int c = threadIdx.x; c < C; c += blockDim.x)
-    bn_finalize_channel(c, tot[2 * c], tot[2 * c + 1], cnt, weight, bias, running_mean, running_var, momentum, eps, save_mean, save_invstd,
-                        scale, shift);
+    bn_finalize_channel(c, tot[2 * c], tot[2 * c + 1], cnt, weight, bias, running_mean, running_var, momentum, eps, scale, shift);
   if (threadIdx.x == 0) {
     if (nbt) *nbt += 1;
     if (s_timeout) atomicAdd(reinterpret_cast<unsigned *>(mine + 8), 1u);
@@ -941,24 +887,30 @@ SFOD_API int sfod_p2p_status(const sfod_p2p_comm_t *comm, uint64_t *exchanges, u
   return SFOD_OK;
 }
 
-SFOD_API int sfod_bn_exchange_finalize_apply(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N,
-                                             int C, int H, int W, double *stats_dev, const sfod_p2p_comm_t *comm, const float *weight,
-                                             const float *bias, float *running_mean, float *running_var, int64_t *num_batches_tracked,
-                                             double momentum, double eps, int fuse_relu, int fuse_maxpool2, float *save_mean,
-                                             float *save_invstd, sfod_stream_t stream) {
-  if (!stats_dev || !comm || N <= 0 || C <= 0 || H <= 0 || W <= 0) return SFOD_ERR_INVALID_ARG;
-  if (!p2p_comm_ok(comm)) return SFOD_ERR_INVALID_ARG;
-  if (2 * C + 1 > kP2PMaxPayload) return SFOD_ERR_UNSUPPORTED;
+// stats_dev layout: [0, 2C) (sum x, sum x^2); [2C] element count (written by phase 1; with [0, 2C) it forms the 2C+1
+// all-reduce payload); [2C + 1] ticket word of the statistics kernel's payload delivery; [2C + 2, ...) float scale / shift
+// scratch of phase 2; [4C, ...) replica totals of the NHWC pass.
+SFOD_API int sfod_bn_finalize_apply(const float *x, const float *pre_bias, const float *residual, float *y, int layout, int N, int C,
+                                    int H, int W, double *stats_dev, const sfod_p2p_comm_t *comm, const float *weight, const float *bias,
+                                    float *running_mean, float *running_var, int64_t *num_batches_tracked, double momentum, double eps,
+                                    int fuse_relu, int fuse_maxpool2, sfod_stream_t stream) {
+  if (!stats_dev || N <= 0 || C <= 0 || H <= 0 || W <= 0) return SFOD_ERR_INVALID_ARG;
+  if (comm && !p2p_comm_ok(comm)) return SFOD_ERR_INVALID_ARG;
+  if (comm && 2 * C + 1 > kP2PMaxPayload) return SFOD_ERR_UNSUPPORTED;
   if (layout != SFOD_NCHW && layout != SFOD_NHWC) return SFOD_ERR_INVALID_ARG;
   if (residual && fuse_maxpool2) return SFOD_ERR_INVALID_ARG;
   if (residual && x && ((reinterpret_cast<uintptr_t>(residual) ^ reinterpret_cast<uintptr_t>(x)) & 15u)) return SFOD_ERR_ALIGNMENT;
   cudaStream_t st = sfod_cu(stream);
   float *scale = reinterpret_cast<float *>(stats_dev + 2 * (size_t)C + 2);
   float *shift = scale + sfod_align_up((size_t)C, 4);
-  bn_exchange_finalize_kernel<<<1, kP2PThreads, 0, st>>>(stats_dev, C, *comm, weight, bias, running_mean, running_var,
-                                                         reinterpret_cast<long long *>(num_batches_tracked), momentum, eps, save_mean,
-                                                         save_invstd, scale, shift);
+  long long *nbt = reinterpret_cast<long long *>(num_batches_tracked);
+  if (comm)   // one CTA: the exchange is a single block that polls for every peer's payload
+    bn_exchange_finalize_kernel<<<1, kP2PThreads, 0, st>>>(stats_dev, C, *comm, weight, bias, running_mean, running_var, nbt, momentum,
+                                                           eps, scale, shift);
+  else
+    bn_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(stats_dev, C, weight, bias, running_mean, running_var, nbt, momentum, eps, scale,
+                                                        shift);
   SFOD_LAUNCH_CHECK();
-  if (!x || !y) return SFOD_OK;
+  if (!x || !y) return SFOD_OK;  // statistics-only mode (AdaBN does not need the normalised output of the last layer)
   return launch_bn_apply(x, pre_bias, residual, y, layout, N, C, H, W, scale, shift, fuse_relu, fuse_maxpool2, st);
 }

@@ -25,7 +25,7 @@ def allreduce_bn_stats(payload: Tensor, num_channels: int, group=None) -> float:
 
 def allreduce_bn_stats_device(payload: Tensor, num_channels: int, group=None) -> None:
     """The same all-reduce without leaving the device: the global count stays in ``payload[2C]`` and is read there by
-    ``sfod_bn_finalize_apply_v2(count_on_device=1)`` -- no ``.item()``, so a multi-GPU AdaBN / teacher forward enqueues all
+    ``sfod_bn_finalize_apply`` -- no ``.item()``, so a multi-GPU AdaBN / teacher forward enqueues all
     of its BN layers without a single host synchronisation."""
     assert payload.dtype == torch.float64 and payload.numel() >= 2 * num_channels + 1
     if dist.is_available() and dist.is_initialized():

@@ -2,7 +2,7 @@
 
 ``PeerStatExchange`` owns one inbox per rank (``sfod_p2p_alloc``), ships its CUDA IPC handle to the other processes of the
 node through ``torch.distributed`` (host plumbing only) and maps theirs; ``ops.bn_train_forward(group=<PeerStatExchange>)``
-then runs ``sfod_bn_exchange_finalize_apply``: the all-reduce of the (sum x, sum x^2, count) payload happens INSIDE the
+then runs ``sfod_bn_finalize_apply`` with the exchange's comm: the all-reduce of the (sum x, sum x^2, count) payload happens INSIDE the
 finalize kernel with P2P stores and flags (csrc/bn.cu), instead of one NCCL all-reduce launch per BN layer
 (``engine/adabn_dist.py``, the baseline it is measured against in ``bench.py``'s ``adabn`` record).
 

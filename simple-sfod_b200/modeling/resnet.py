@@ -9,7 +9,7 @@ normalisation path of the teacher / AdaBN forwards (train() under no_grad):
 
 * ``conv -> BN -> ReLU`` runs the two native BN kernels (statistics 4 B/element, fused normalise+ReLU in place 8 B/element);
 * the bottleneck tail ``conv3 -> BN``, ``out += shortcut``, ``relu_`` -- three elementwise passes (28 B/element) in
-  detectron2's ``BottleneckBlock.forward`` -- is ONE pass (``residual`` fusion of ``sfod_bn_finalize_apply_v2``, 12 B/element);
+  detectron2's ``BottleneckBlock.forward`` -- is ONE pass (``residual`` fusion of ``sfod_bn_finalize_apply``, 12 B/element);
 * the frozen stem and res2 (``FREEZE_AT 2`` turns their 11 norm layers into ``FrozenBatchNorm2d``) use the same fused pass with
   coefficients from the running statistics (``sfod_bn_frozen_apply``).
 

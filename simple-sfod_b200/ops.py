@@ -697,6 +697,20 @@ class EmaPlan:
 BN_P2P_TAIL_PUSH = int(os.environ.get("SFOD_P2P_TAIL_PUSH", "0"))
 
 
+def _ptr(t: Optional[Tensor]) -> Optional[int]:
+    return t.data_ptr() if t is not None else None
+
+
+def _residual_like(residual: Tensor, xin: Tensor, layout: int) -> Tensor:
+    """``residual`` in the memory layout of ``xin`` (the fused residual add reads both with the same indexing)."""
+    res, rl = _layout_of(residual.detach())
+    if res.shape != xin.shape or res.dtype != torch.float32:
+        raise ValueError("residual must have the shape and dtype of x")
+    if rl != layout:
+        res = res.contiguous(memory_format=torch.channels_last if layout == NHWC else torch.contiguous_format)
+    return res
+
+
 def bn_train_forward(x: Tensor, weight: Optional[Tensor], bias: Optional[Tensor], running_mean: Optional[Tensor],
                      running_var: Optional[Tensor], num_batches_tracked: Optional[Tensor], momentum: float = 0.1,
                      eps: float = 1e-5, fuse_relu: bool = False, inplace: bool = False, group=None,
@@ -719,15 +733,9 @@ def bn_train_forward(x: Tensor, weight: Optional[Tensor], bias: Optional[Tensor]
         pb = pre_bias.detach()
         if pb.dtype != torch.float32 or pb.numel() != Cc or not pb.is_contiguous():
             raise ValueError("pre_bias must be a contiguous float32 tensor with one entry per channel")
-    res = None
-    if residual is not None:
-        if fuse_maxpool:
-            raise ValueError("residual and fuse_maxpool are mutually exclusive")
-        res, rl = _layout_of(residual.detach())
-        if res.shape != xin.shape or res.dtype != torch.float32:
-            raise ValueError("residual must have the shape and dtype of x")
-        if rl != layout:
-            res = res.contiguous(memory_format=torch.channels_last if layout == NHWC else torch.contiguous_format)
+    if residual is not None and fuse_maxpool:
+        raise ValueError("residual and fuse_maxpool are mutually exclusive")
+    res = _residual_like(residual, xin, layout) if residual is not None else None
     L = _lib.lib()
     with torch.cuda.device(dev):
         stats = torch.empty((L.sfod_bn_stats_bytes(Cc) // 8,), dtype=torch.float64, device=dev)
@@ -736,37 +744,27 @@ def bn_train_forward(x: Tensor, weight: Optional[Tensor], bias: Optional[Tensor]
             # activation fits L2: statistics -> grid barrier -> normalise in ONE cooperative launch (second read of x from L2)
             y = xin if inplace else torch.empty_like(xin)
             with _timed("bn_train_fused_res" if res is not None else "bn_train_fused"):
-                rc = L.sfod_bn_train_fused(xin.data_ptr(), pb.data_ptr() if pb is not None else None,
-                                           res.data_ptr() if res is not None else None, y.data_ptr(), N, Cc, H, W, stats.data_ptr(),
-                                           weight.data_ptr() if weight is not None else None, bias.data_ptr() if bias is not None else None,
-                                           running_mean.data_ptr() if running_mean is not None else None,
-                                           running_var.data_ptr() if running_var is not None else None,
-                                           num_batches_tracked.data_ptr() if num_batches_tracked is not None else None,
+                rc = L.sfod_bn_train_fused(xin.data_ptr(), _ptr(pb), _ptr(res), y.data_ptr(), N, Cc, H, W, stats.data_ptr(),
+                                           _ptr(weight), _ptr(bias), _ptr(running_mean), _ptr(running_var), _ptr(num_batches_tracked),
                                            float(momentum), float(eps), int(fuse_relu), _stream(dev))
             if rc == 0:
                 return y
             if rc != 3:   # SFOD_ERR_UNSUPPORTED: no cooperative grid -> the two-phase path below
                 check(rc, "sfod_bn_train_fused")
-        peer = None
+        comm = None
         if group is not None:
             from .engine.p2p import PeerStatExchange
             if isinstance(group, PeerStatExchange):
-                peer = group   # the all-reduce happens inside the statistics / finalize kernels, over NVLink peer memory
-                if Cc > peer.max_channels:
-                    raise ValueError(f"PeerStatExchange carries at most {peer.max_channels} channels per layer")
+                # the all-reduce happens inside the finalize kernel (or the statistics kernel's last CTA), over NVLink peer memory
+                if Cc > group.max_channels:
+                    raise ValueError(f"PeerStatExchange carries at most {group.max_channels} channels per layer")
+                comm = C.byref(group.comm)
         with _timed("bn_partial_stats"):
-            if peer is not None and BN_P2P_TAIL_PUSH:
-                check(L.sfod_bn_partial_stats_p2p(xin.data_ptr(), pb.data_ptr() if pb is not None else None, layout, N, Cc, H * W,
-                                                  stats.data_ptr(), C.byref(peer.comm), _stream(dev)), "sfod_bn_partial_stats_p2p")
-            else:
-                check(L.sfod_bn_partial_stats(xin.data_ptr(), pb.data_ptr() if pb is not None else None, layout, N, Cc, H * W,
-                                              stats.data_ptr(), _stream(dev)), "sfod_bn_partial_stats")
-        on_device = 0
-        if group is not None:
-            if peer is None:
-                from .engine.adabn_dist import allreduce_bn_stats_device
-                allreduce_bn_stats_device(stats, Cc, group=group if group is not True else None)   # payload [0, 2C] incl. the count
-                on_device = 1
+            check(L.sfod_bn_partial_stats(xin.data_ptr(), _ptr(pb), layout, N, Cc, H * W, stats.data_ptr(),
+                                          comm if BN_P2P_TAIL_PUSH else None, _stream(dev)), "sfod_bn_partial_stats")
+        if group is not None and comm is None:
+            from .engine.adabn_dist import allreduce_bn_stats_device
+            allreduce_bn_stats_device(stats, Cc, group=group if group is not True else None)   # payload [0, 2C] incl. the count
         y = None
         if compute_output:
             if fuse_maxpool:
@@ -774,32 +772,15 @@ def bn_train_forward(x: Tensor, weight: Optional[Tensor], bias: Optional[Tensor]
                 y = torch.empty((N, Cc, H // 2, W // 2), dtype=torch.float32, device=dev, memory_format=fmt)
             else:
                 y = xin if inplace else torch.empty_like(xin)
-        if peer is not None:
-            with _timed("bn_exchange_finalize_apply"):
-                check(L.sfod_bn_exchange_finalize_apply(xin.data_ptr() if compute_output else None, pb.data_ptr() if pb is not None else None,
-                                                        res.data_ptr() if (res is not None and compute_output) else None,
-                                                        y.data_ptr() if y is not None else None, layout, N, Cc, H, W, stats.data_ptr(),
-                                                        C.byref(peer.comm),
-                                                        weight.data_ptr() if weight is not None else None,
-                                                        bias.data_ptr() if bias is not None else None,
-                                                        running_mean.data_ptr() if running_mean is not None else None,
-                                                        running_var.data_ptr() if running_var is not None else None,
-                                                        num_batches_tracked.data_ptr() if num_batches_tracked is not None else None,
-                                                        float(momentum), float(eps), int(fuse_relu), int(fuse_maxpool), None, None,
-                                                        _stream(dev)), "sfod_bn_exchange_finalize_apply")
-            return y
-        with _timed("bn_finalize_apply_pool" if fuse_maxpool else ("bn_finalize_apply_res" if res is not None else "bn_finalize_apply")):
-            check(L.sfod_bn_finalize_apply_v2(xin.data_ptr() if compute_output else None, pb.data_ptr() if pb is not None else None,
-                                              res.data_ptr() if (res is not None and compute_output) else None,
-                                              y.data_ptr() if y is not None else None, layout, N, Cc, H, W, stats.data_ptr(),
-                                              float(N * H * W), on_device,
-                                              weight.data_ptr() if weight is not None else None,
-                                              bias.data_ptr() if bias is not None else None,
-                                              running_mean.data_ptr() if running_mean is not None else None,
-                                              running_var.data_ptr() if running_var is not None else None,
-                                              num_batches_tracked.data_ptr() if num_batches_tracked is not None else None,
-                                              float(momentum), float(eps), int(fuse_relu), int(fuse_maxpool), None, None, _stream(dev)),
-                  "sfod_bn_finalize_apply_v2")
+        if comm is not None:
+            tag = "bn_exchange_finalize_apply"
+        else:
+            tag = "bn_finalize_apply_pool" if fuse_maxpool else ("bn_finalize_apply_res" if res is not None else "bn_finalize_apply")
+        with _timed(tag):
+            check(L.sfod_bn_finalize_apply(xin.data_ptr() if compute_output else None, _ptr(pb), _ptr(res) if compute_output else None,
+                                           _ptr(y), layout, N, Cc, H, W, stats.data_ptr(), comm, _ptr(weight), _ptr(bias),
+                                           _ptr(running_mean), _ptr(running_var), _ptr(num_batches_tracked), float(momentum), float(eps),
+                                           int(fuse_relu), int(fuse_maxpool), _stream(dev)), "sfod_bn_finalize_apply")
     return y
 
 
@@ -811,20 +792,13 @@ def bn_frozen_forward(x: Tensor, weight: Optional[Tensor], bias: Optional[Tensor
     if xin.dtype != torch.float32:
         raise TypeError("bn_frozen_forward computes in float32")
     N, Cc, H, W = xin.shape
-    res = None
-    if residual is not None:
-        res, rl = _layout_of(residual.detach())
-        if res.shape != xin.shape or res.dtype != torch.float32:
-            raise ValueError("residual must have the shape and dtype of x")
-        if rl != layout:
-            res = res.contiguous(memory_format=torch.channels_last if layout == NHWC else torch.contiguous_format)
+    res = _residual_like(residual, xin, layout) if residual is not None else None
     L = _lib.lib()
     with torch.cuda.device(dev):
         scratch = torch.empty((L.sfod_bn_frozen_scratch_bytes(Cc),), dtype=torch.uint8, device=dev)
         y = xin if inplace else torch.empty_like(xin)
         with _timed("bn_frozen_apply"):
-            check(L.sfod_bn_frozen_apply(xin.data_ptr(), res.data_ptr() if res is not None else None, y.data_ptr(), layout, N, Cc, H, W,
-                                         weight.data_ptr() if weight is not None else None, bias.data_ptr() if bias is not None else None,
+            check(L.sfod_bn_frozen_apply(xin.data_ptr(), _ptr(res), y.data_ptr(), layout, N, Cc, H, W, _ptr(weight), _ptr(bias),
                                          running_mean.data_ptr(), running_var.data_ptr(), float(eps), int(fuse_relu),
                                          scratch.data_ptr(), _stream(dev)), "sfod_bn_frozen_apply")
     return y

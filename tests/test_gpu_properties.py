@@ -117,7 +117,7 @@ def test_ema_fixed_points_on_vgg_state(ops, cuda_device):
         assert torch.equal(v, want), k
 
 
-def test_bn_statistics_full_size(ops, cuda_device):
+def test_bn_statistics_full_size_abi_v2(ops, cuda_device):
     N, C, H, W = 8, 64, 600, 1200
     g = torch.Generator(device=cuda_device).manual_seed(2)
     x = torch.randn(N, C, H, W, device=cuda_device, generator=g) * 2 + torch.linspace(-30, 30, C, device=cuda_device).view(1, C, 1, 1)
@@ -132,7 +132,7 @@ def test_bn_statistics_full_size(ops, cuda_device):
     L = sfod_b200._lib.lib()
     def raw(t):
         st = torch.empty(L.sfod_bn_stats_bytes(C) // 8, dtype=torch.float64, device=cuda_device)
-        sfod_b200._lib.check(L.sfod_bn_partial_stats(t.data_ptr(), None, 0, t.shape[0], C, H * W, st.data_ptr(),
+        sfod_b200._lib.check(L.sfod_bn_partial_stats(t.data_ptr(), None, 0, t.shape[0], C, H * W, st.data_ptr(), None,
                                                      torch.cuda.current_stream().cuda_stream))
         return st[: 2 * C].clone()
     whole, a, b = raw(x), raw(x[:4].contiguous()), raw(x[4:].contiguous())
@@ -201,7 +201,7 @@ def test_adabn_statistic_allreduce_nccl_two_gpus(tmp_path):
 
 @pytest.mark.parametrize("world", [3, 6])   # all 8 slots are exercised by the 8-process bench self-check (profiles/r2s_*)
 def test_peer_statistic_exchange_local_ring_matches_concatenated_batch(cuda_device, world):
-    """The NVLink peer-memory all-reduce of the BN statistics (sfod_bn_exchange_finalize_apply), with the ranks emulated as
+    """The NVLink peer-memory all-reduce of the BN statistics (sfod_bn_finalize_apply with a comm), with the ranks emulated as
     streams of ONE GPU (their inboxes are plain allocations in this process): every rank must end with the running statistics
     and the normalised output of nn.BatchNorm2d on the concatenated batch, the exchanged totals must be bit-identical on all
     ranks, and repeated exchanges (slot parity, device-side epoch counter) must keep working without a host reset."""

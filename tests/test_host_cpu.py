@@ -39,10 +39,10 @@ def test_library_exports_every_declared_symbol():
     assert {e for e in exported if e.startswith("sfod_")} == declared
 
 
-def test_host_only_entry_points():
+def test_host_only_entry_points_abi_v2():
     L = _lib.lib()
     launches = L.sfod_debug_launch_count()                      # non-zero when GPU tests ran earlier in this process
-    assert L.sfod_abi_version() == 1
+    assert L.sfod_abi_version() == 2
     # the ctypes mirrors of the parameter structs have the C layout (sizeof as compiled into the library)
     for which, mirror in enumerate((_lib.EmaTensor, _lib.RpnParams, _lib.FrcnnParams, _lib.P2PComm, _lib.JitterParams, _lib.EraseParams)):
         assert L.sfod_abi_sizeof(which) == C.sizeof(mirror), (which, mirror.__name__, L.sfod_abi_sizeof(which), C.sizeof(mirror))
@@ -61,13 +61,13 @@ def test_host_only_entry_points():
     comm = _lib.P2PComm(); comm.rank, comm.world = 0, 2
     comm.inbox[0] = 0x1000                                                                                # inbox[1] missing
     a = [None] * 4 + [0, 8, 64, 20, 20, 0x2000]
-    tail = [None] * 5 + [0.1, 1e-5, 0, 0, None, None, None]
-    assert L.sfod_bn_exchange_finalize_apply(*a, C.byref(comm), *tail) == 1
+    tail = [None] * 5 + [0.1, 1e-5, 0, 0, None]
+    assert L.sfod_bn_finalize_apply(*a, C.byref(comm), *tail) == 1
     comm.inbox[1] = 0x3000; comm.world = 9
-    assert L.sfod_bn_exchange_finalize_apply(*a, C.byref(comm), *tail) == 1
+    assert L.sfod_bn_finalize_apply(*a, C.byref(comm), *tail) == 1
     comm.world = 2
     a[6] = 2052                                                                                           # C beyond the payload slot
-    assert L.sfod_bn_exchange_finalize_apply(*a, C.byref(comm), *tail) == 3
+    assert L.sfod_bn_finalize_apply(*a, C.byref(comm), *tail) == 3
     assert L.sfod_p2p_status(C.byref(_lib.P2PComm()), None, None) == 1 and L.sfod_p2p_open(None, None) == 1
     p = _lib.RpnParams(); p.N, p.HWA, p.pre_nms_topk, p.post_nms_topk = 8, 9990, 12000, 2000
     assert L.sfod_rpn_select_workspace_bytes(C.byref(p)) > 8 * 9990 * 157 * 8
@@ -83,6 +83,23 @@ def test_host_only_entry_points():
     arr[1].dtype = 7
     assert L.sfod_ema_plan_build(arr, 2, buf, len(buf)) == 3    # SFOD_ERR_UNSUPPORTED
     assert L.sfod_debug_launch_count() == launches              # nothing was launched by any of the above
+
+
+def test_binding_refuses_a_library_of_another_abi(monkeypatch):
+    """A library built from another revision of the header would take the binding's argument lists unchecked."""
+    monkeypatch.setattr(_lib, "_lib", None)
+    monkeypatch.setattr(_lib, "ABI_VERSION", 1)
+    with pytest.raises(_lib.SfodLibraryError, match="ABI version 2, this binding expects 1"):
+        _lib.lib()
+    monkeypatch.undo()
+
+    class P2PComm4(C.Structure):                                  # a mirror written for four ranks instead of eight
+        _fields_ = [("rank", C.c_int32), ("world", C.c_int32), ("inbox", C.c_void_p * 4)]
+    monkeypatch.setattr(_lib, "_lib", None)
+    monkeypatch.setattr(_lib, "ABI_STRUCTS", _lib.ABI_STRUCTS[:3] + (P2PComm4,) + _lib.ABI_STRUCTS[4:])
+    with pytest.raises(_lib.SfodLibraryError, match="struct 3 has 72 bytes, its ctypes mirror P2PComm4 40"):
+        _lib.lib()
+    assert _lib._lib is None
 
 
 def test_product_never_imports_oracle_and_has_no_cpu_fallback():
