@@ -49,7 +49,7 @@ enum sfod_dtype { SFOD_F32 = 0, SFOD_I64 = 1, SFOD_U8 = 2 };
 /* Changes whenever an entry point keeps its name but changes its arguments; a binding refuses a library of another version. */
 int sfod_abi_version(void);
 /* sizeof() of the parameter structs as this library was compiled (which: 0 sfod_ema_tensor, 1 sfod_rpn_params,
- * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params; 0 for anything else) -- lets a foreign
+ * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params, 6 sfod_resize_image; 0 for anything else) -- lets a foreign
  * binding (ctypes / cffi struct mirrors) check its layout against the C one before the first call. */
 size_t sfod_abi_sizeof(int which);
 const char *sfod_status_string(int status);
@@ -408,6 +408,38 @@ typedef struct sfod_erase_params {
  * ToPILImage leave in the rectangle. */
 int sfod_random_erase(uint8_t *images, int N, int H, int W, const sfod_erase_params *params_dev, const float *noise,
                       uint64_t seed, sfod_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------------------------------
+ * Weak augmentation of the input on the device (SURVEY.md 8f rank 3): detectron2's ResizeShortestEdge + RandomFlip, the
+ * augmentations the reference's data mapper applies before the strong chain (reference
+ * daod/data/mappers/two_crop_augmentation_mapper.py, `T.apply_augmentations(self.augmentation, aug_input)` with the list of
+ * detectron2 build_augmentation).  For uint8 images detectron2's ResizeTransform.apply_image is
+ * `Image.fromarray(img).resize((new_w, new_h), Image.BILINEAR)`; HFlipTransform is `np.flip(img, axis=1)` after it.
+ * This call reproduces Pillow's 8-bit resampler (src/libImaging/Resample.c) bit for bit: horizontal pass over the input rows the
+ * vertical taps use, rounded to a uint8 intermediate, then the vertical pass; every output is
+ * clip8(2^21 + sum in[xmin + k] * tap[k]) in int32 with 22 fraction bits.  The taps come from the caller (the host computes them
+ * in double exactly as Pillow does: simple-sfod_b200/ops.py::pil_resize_coeffs).
+ * Per image one record; the source is read through three byte strides, so HWC (stride_px = 3, stride_ch = 1) and CHW planes
+ * (stride_px = 1, stride_ch = H * W, i.e. a permuted view) take the same path.  The result is written as CHW planes
+ * (3, out_h, out_w) at out + out_offset (the mapper's HWC -> CHW transpose is fused), mirrored horizontally when hflip != 0.
+ * A coefficient table (int32, at coeffs + k*_offset) holds out (xmin, xmax) pairs followed by out x k*_size taps, zero-padded
+ * to k*_size = 2 * ceil(max(in / out, 1)) + 1.  Down-scales up to 4 per axis (k*_size <= 9) and any up-scale are supported. */
+typedef struct sfod_resize_image {
+  const uint8_t *src;                         /* device pointer: pixel (0, 0), channel 0 */
+  int64_t stride_row, stride_px, stride_ch;   /* bytes */
+  int32_t in_h, in_w, out_h, out_w;
+  int64_t out_offset;                         /* bytes from `out` to this image's (3, out_h, out_w) planes */
+  int32_t hflip;                              /* != 0: write column x to out_w - 1 - x */
+  int32_t kx_offset, kx_size;                 /* horizontal table: int32 offset into coeffs, taps per output column */
+  int32_t ky_offset, ky_size;                 /* vertical table */
+  int32_t reserved;
+} sfod_resize_image;
+/* One launch for the whole batch.  records_dev: N records in DEVICE memory; max_out_h / max_out_w / max_ksize: maxima over the
+ * records (they size the grid and the shared-memory tiles; a record beyond them is skipped, its output left unwritten).
+ * SFOD_ERR_INVALID_ARG for null pointers, N < 0, non-positive maxima, or max_out_h * max_out_w beyond an int32 plane index;
+ * SFOD_ERR_UNSUPPORTED for max_ksize > 9 (a down-scale beyond 4). */
+int sfod_resize_pil(const sfod_resize_image *records_dev, int N, const int32_t *coeffs_dev, uint8_t *out, int max_out_h,
+                    int max_out_w, int max_ksize, sfod_stream_t stream);
 
 #ifdef __cplusplus
 }

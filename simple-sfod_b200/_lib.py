@@ -32,6 +32,13 @@ class EraseParams(C.Structure):
     _fields_ = [("n_rects", C.c_int32), ("rect", (C.c_int32 * 4) * 4)]
 
 
+class ResizeImage(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("stride_row", C.c_int64), ("stride_px", C.c_int64), ("stride_ch", C.c_int64),
+                ("in_h", C.c_int32), ("in_w", C.c_int32), ("out_h", C.c_int32), ("out_w", C.c_int32), ("out_offset", C.c_int64),
+                ("hflip", C.c_int32), ("kx_offset", C.c_int32), ("kx_size", C.c_int32), ("ky_offset", C.c_int32),
+                ("ky_size", C.c_int32), ("reserved", C.c_int32)]
+
+
 class RpnParams(C.Structure):
     _fields_ = [("N", C.c_int), ("HWA", C.c_int), ("A", C.c_int), ("Hf", C.c_int), ("Wf", C.c_int), ("stride", C.c_int),
                 ("anchor_offset", C.c_float), ("weights", C.c_float * 4), ("scale_clamp", C.c_float),
@@ -56,7 +63,7 @@ class P2PComm(C.Structure):
 
 # sfod_abi_version() of the library this binding is written for, and the struct mirrors in the order of sfod_abi_sizeof(which)
 ABI_VERSION = 2
-ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams)
+ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams, ResizeImage)
 
 
 # name -> (restype, argtypes); every symbol include/sfod_b200.h declares
@@ -99,6 +106,7 @@ SIGNATURES = {
     "sfod_gaussian_blur": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "sfod_gaussian_blur_pil": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "sfod_random_erase": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_uint64, c_ptr]),
+    "sfod_resize_pil": (C.c_int, [c_ptr, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
     "sfod_subsample_labels": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_uint64, c_ptr, c_ptr, c_ptr]),
     "sfod_bn_stats_bytes": (C.c_size_t, [C.c_int]),
     "sfod_bn_partial_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, C.POINTER(P2PComm), c_ptr]),

@@ -84,7 +84,8 @@ _DEFAULTS = {
                          "TRAIN_ON_PRED_BOXES": False, "USE_FED_LOSS": False, "USE_SIGMOID_CE": False},
         "RESNETS": {"DEPTH": 50, "OUT_FEATURES": ["res4"], "NORM": "FrozenBN"},
     },
-    "INPUT": {"MIN_SIZE_TRAIN": (800,), "MAX_SIZE_TRAIN": 1333, "MIN_SIZE_TEST": 800, "MAX_SIZE_TEST": 1333, "FORMAT": "BGR"},
+    "INPUT": {"MIN_SIZE_TRAIN": (800,), "MIN_SIZE_TRAIN_SAMPLING": "choice", "MAX_SIZE_TRAIN": 1333, "MIN_SIZE_TEST": 800,
+              "MAX_SIZE_TEST": 1333, "RANDOM_FLIP": "horizontal", "FORMAT": "BGR"},
     "VIS_PERIOD": 0,
     "TEST": {"DETECTIONS_PER_IMAGE": 100},
     "SOLVER": {"IMS_PER_BATCH": 16, "IMS_PER_BATCH_TARGET": 16},

@@ -425,6 +425,7 @@ SFOD_API size_t sfod_abi_sizeof(int which) {
     case 3: return sizeof(sfod_p2p_comm);
     case 4: return sizeof(sfod_jitter_params);
     case 5: return sizeof(sfod_erase_params);
+    case 6: return sizeof(sfod_resize_image);
     default: return 0;
   }
 }

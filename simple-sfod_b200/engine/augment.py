@@ -1,4 +1,12 @@
-"""Strong augmentation of the student's batch on the GPU (SURVEY.md 8f rank 3).
+"""Weak and strong augmentation of the input batch on the GPU (SURVEY.md 8f rank 3).
+
+Weak: the reference's mapper first applies detectron2's ``build_augmentation(cfg, is_train)`` -- ResizeShortestEdge, then (training)
+RandomFlip -- to every image; the teacher consumes this weak image and the strong chain below runs on it.  ``draw_weak_params``
+draws the decisions with the same numpy calls in the same order as detectron2's ``get_transform``s, ``weak_augment`` does the
+pixel work in one launch (``ops.resize_pil``: Pillow's BILINEAR resize + flip + HWC -> CHW, bit for bit) and
+``apply_weak_to_boxes`` maps annotation boxes as ``transform_instance_annotations`` does.
+
+Strong:
 
 The reference builds, per image and on the CPU (PIL), reference daod/data/detection_utils.py:7-37:
 
@@ -14,12 +22,14 @@ instead of ~10 PIL passes per image on one CPU core).  Images are RGB uint8 (N, 
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Sequence, Tuple, Union
 
+import numpy as np
 import torch
 from torch import Tensor
 
 from .. import ops
+from ..config import CfgNode, get_cfg
 
 JITTER = dict(brightness=(0.6, 1.4), contrast=(0.6, 1.4), saturation=(0.6, 1.4), hue=(-0.1, 0.1), p=0.8)   # ColorJitter(0.4, 0.4, 0.4, 0.1)
 GRAYSCALE_P = 0.2
@@ -96,3 +106,94 @@ def strong_augment(images: Tensor, params: Optional[List[Dict]] = None, generato
             seed = int(torch.randint(0, 2 ** 62, (1,), generator=generator if generator is not None else torch.default_generator))
         ops.random_erase_(x, [p["rects"] for p in params], noise=noise, seed=seed)
     return x
+
+
+# ------------------------------------------------------------------------------------------------------------- weak augmentation
+def _resize_shortest_edge_shape(h: int, w: int, size: int, max_size: int) -> Tuple[int, int]:
+    """detectron2 ResizeShortestEdge.get_output_shape."""
+    size = size * 1.0
+    scale = size / min(h, w)
+    if h < w:
+        newh, neww = size, scale * w
+    else:
+        newh, neww = scale * h, size
+    if max(newh, neww) > max_size:
+        scale = max_size * 1.0 / max(newh, neww)
+        newh = newh * scale
+        neww = neww * scale
+    return int(newh + 0.5), int(neww + 0.5)
+
+
+def draw_weak_params(image_sizes: Sequence[Tuple[int, int]], cfg: CfgNode, is_train: bool = True,
+                     rng: Optional[np.random.RandomState] = None) -> List[Dict]:
+    """Per image ``{"size": (h, w), "hflip": bool}``: the decisions of detectron2's ``build_augmentation(cfg, is_train)`` --
+    ``ResizeShortestEdge(MIN_SIZE_*, MAX_SIZE_*, sampling)`` and, in training, ``RandomFlip`` -- drawn with the same numpy calls in
+    the same order as their ``get_transform``s (per image: the short edge, then the flip on the resized image).  ``rng=None``
+    draws from numpy's global state, as detectron2 does."""
+    r = np.random if rng is None else rng
+    if is_train:
+        short, max_size, style = cfg.INPUT.MIN_SIZE_TRAIN, cfg.INPUT.MAX_SIZE_TRAIN, cfg.INPUT.get("MIN_SIZE_TRAIN_SAMPLING", "choice")
+        flip = cfg.INPUT.get("RANDOM_FLIP", "horizontal")
+    else:
+        short, max_size, style, flip = cfg.INPUT.MIN_SIZE_TEST, cfg.INPUT.MAX_SIZE_TEST, "choice", "none"
+    if style not in ("range", "choice"):
+        raise ValueError(f"MIN_SIZE_TRAIN_SAMPLING {style!r}")
+    if flip not in ("horizontal", "none"):
+        raise NotImplementedError(f"RANDOM_FLIP {flip!r}: only 'horizontal' and 'none' are supported")
+    if isinstance(short, int):
+        short = (short, short)
+    if style == "range" and len(short) != 2:
+        raise ValueError("MIN_SIZE_TRAIN_SAMPLING 'range' needs two sizes")
+    out = []
+    for h, w in image_sizes:
+        size = r.randint(short[0], short[1] + 1) if style == "range" else r.choice(short)
+        if size == 0:                                                    # NoOpTransform
+            newh, neww = int(h), int(w)
+        else:
+            newh, neww = _resize_shortest_edge_shape(int(h), int(w), size, max_size)
+        do_flip = bool(r.uniform(0, 1.0, []) < 0.5) if flip == "horizontal" else False   # RandomFlip._rand_range() < prob
+        out.append({"size": (newh, neww), "hflip": do_flip})
+    return out
+
+
+def weak_augment(images: Union[Tensor, Sequence[Tensor]], params: Optional[List[Dict]] = None, cfg: Optional[CfgNode] = None,
+                 is_train: bool = True, rng: Optional[np.random.RandomState] = None) -> Tuple[Union[Tensor, List[Tensor]], List[Dict]]:
+    """Resize (+ flip) a batch of decoded uint8 RGB images on the GPU: ``images`` is a (N, H, W, 3) tensor or a list of (H, W, 3)
+    CUDA tensors or views (``x.permute(1, 2, 0)`` for a CHW image).  Without ``params`` the decisions are drawn by
+    ``draw_weak_params`` from ``cfg`` (detectron2's defaults, ``config.get_cfg()``, when None).  Returns the CHW weak images -- a
+    (N, 3, h, w) tensor when all sizes agree, otherwise a list -- and the parameters used."""
+    imgs = list(images.unbind(0)) if isinstance(images, Tensor) else list(images)
+    if params is None:
+        params = draw_weak_params([(int(im.shape[0]), int(im.shape[1])) for im in imgs], cfg if cfg is not None else get_cfg(),
+                                  is_train, rng)
+    out = ops.resize_pil(images, [p["size"] for p in params], [p["hflip"] for p in params])
+    return out, params
+
+
+def apply_weak_to_boxes(boxes_xyxy, image_size: Tuple[int, int], param: Dict) -> np.ndarray:
+    """detectron2 ``transform_instance_annotations`` for the weak transforms: each transform maps the four corners of every box
+    (resize ``x * (new_w / w)``, ``y * (new_h / h)``; flip ``x -> new_w - x``) and takes their min / max; the result is clipped
+    to ``[0, new size]``.  float64 arithmetic; float32 result (what ``Boxes`` stores).  ``image_size`` = the original (h, w)."""
+    h, w = int(image_size[0]), int(image_size[1])
+    newh, neww = (int(v) for v in param["size"])
+    box = np.asarray(boxes_xyxy, dtype=np.float64).reshape(-1, 4)
+    idxs = np.array([(0, 1), (2, 1), (0, 3), (2, 3)]).flatten()
+
+    def apply_box(b, fn):
+        coords = fn(b[:, idxs].reshape(-1, 2)).reshape((-1, 4, 2))
+        return np.concatenate((coords.min(axis=1), coords.max(axis=1)), axis=1)
+
+    def resize(c):
+        c[:, 0] = c[:, 0] * (neww * 1.0 / w)
+        c[:, 1] = c[:, 1] * (newh * 1.0 / h)
+        return c
+
+    def hflip(c):
+        c[:, 0] = neww - c[:, 0]
+        return c
+
+    box = apply_box(box, resize)
+    if param["hflip"]:
+        box = apply_box(box, hflip)
+    box = np.minimum(box.clip(min=0), [neww, newh, neww, newh])
+    return box.astype(np.float32)

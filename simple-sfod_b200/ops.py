@@ -18,7 +18,7 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from ._lib import EmaTensor, EraseParams, FrcnnParams, JitterParams, RpnParams, check
+from ._lib import EmaTensor, EraseParams, FrcnnParams, JitterParams, ResizeImage, RpnParams, check
 
 NCHW, NHWC = 0, 1
 DT_F32, DT_I64, DT_U8 = 0, 1, 2   # enum sfod_dtype
@@ -962,3 +962,141 @@ def random_erase_(images: Tensor, rects: Sequence[Sequence[Tuple[int, int, int, 
         check(_lib.lib().sfod_random_erase(images.data_ptr(), N, H, W, rec.data_ptr(), noise.data_ptr() if noise is not None else None,
                                            int(seed) & _MASK64, _stream(dev)), "sfod_random_erase")
     return images
+
+
+# ----------------------------------------------------------------------------------------------- weak augmentation (8f rank 3)
+RESIZE_MAX_KSIZE = 9          # ksize = 2 * ceil(max(in / out, 1)) + 1: down-scales up to 4 per axis
+
+
+def pil_resize_coeffs(in_size: int, out_size: int) -> Tuple[Tensor, Tensor]:
+    """Bounds ``(out, 2)`` int32 ``[xmin, xmax]`` and taps ``(out, ksize)`` int32 (zero past ``xmax``) of Pillow's 8-bit BILINEAR
+    resampler along one axis (Pillow src/libImaging/Resample.c: ``precompute_coeffs`` + ``normalize_coeffs_8bpc``), in Python
+    floats (C doubles) and in Pillow's order: the weights are summed sequentially before they are normalised."""
+    in_size, out_size = int(in_size), int(out_size)
+    if in_size <= 0 or out_size <= 0:
+        raise ValueError("sizes must be positive")
+    scale = float(in_size) / out_size
+    fs = max(scale, 1.0)
+    support = 1.0 * fs
+    ksize = int(math.ceil(support)) * 2 + 1
+    ss = 1.0 / fs
+    bounds = [[0, 0] for _ in range(out_size)]
+    taps = [[0] * ksize for _ in range(out_size)]
+    for xx in range(out_size):
+        center = (xx + 0.5) * scale
+        xmin = max(int(center - support + 0.5), 0)
+        xmax = min(int(center + support + 0.5), in_size) - xmin
+        w = []
+        for x in range(xmax):
+            t = abs((x + xmin - center + 0.5) * ss)
+            w.append(1.0 - t if t < 1.0 else 0.0)
+        ww = 0.0
+        for v in w:
+            ww += v
+        for x, v in enumerate(w):
+            if ww != 0.0:
+                v = v / ww
+            taps[xx][x] = int(-0.5 + v * (1 << 22)) if v < 0 else int(0.5 + v * (1 << 22))
+        bounds[xx] = [xmin, xmax]
+    return torch.tensor(bounds, dtype=torch.int32), torch.tensor(taps, dtype=torch.int32)
+
+
+# device-resident coefficient tables: one growing int32 arena per device, every (in, out) pair uploaded once.  The kernel addresses
+# the tables by int32 offsets into the arena; a grown arena copies the old tables to the same offsets, and the old one stays alive
+# (a launch enqueued earlier may still read it).
+_resize_arena: Dict[int, dict] = {}
+
+
+def _resize_table(dev: torch.device, in_size: int, out_size: int) -> Tuple[int, int]:
+    """-> (offset into the device arena, ksize) of the table of one axis."""
+    idx = dev.index if dev.index is not None else torch.cuda.current_device()
+    a = _resize_arena.setdefault(idx, {"buf": None, "used": 0, "index": {}, "old": []})
+    hit = a["index"].get((in_size, out_size))
+    if hit is not None:
+        return hit
+    bounds, taps = pil_resize_coeffs(in_size, out_size)
+    table = torch.cat([bounds.reshape(-1), taps.reshape(-1)])
+    off, n = a["used"], table.numel()
+    if a["buf"] is None or off + n > a["buf"].numel():
+        grown = torch.empty(max(2 * (off + n), 1 << 16), dtype=torch.int32, device=dev)
+        if a["buf"] is not None:
+            grown[:off].copy_(a["buf"][:off])
+            a["old"].append(a["buf"])
+        a["buf"] = grown
+    a["buf"][off:off + n].copy_(table)
+    a["used"] = off + n
+    a["index"][(in_size, out_size)] = (off, int(taps.shape[1]))
+    return off, int(taps.shape[1])
+
+
+class ResizePlan:
+    """Host-side part of one ``resize_pil`` call: the per-image records (uploaded to the device), the output layout and the launch
+    geometry.  ``launch(out)`` enqueues the kernel; a plan can be launched again while its inputs and tables stay alive."""
+
+    def __init__(self, images: Union[Tensor, Sequence[Tensor]], sizes: Sequence[Tuple[int, int]], hflip: Optional[Sequence[bool]] = None):
+        imgs = list(images.unbind(0)) if isinstance(images, Tensor) else list(images)
+        if isinstance(images, Tensor) and images.dim() != 4:
+            raise ValueError("a batched input must be (N, H, W, 3)")
+        if not imgs:
+            raise ValueError("empty image batch")
+        dev = _require_cuda(*imgs)
+        N = len(imgs)
+        sizes = [(int(h), int(w)) for h, w in sizes]
+        flips = [False] * N if hflip is None else [bool(f) for f in hflip]
+        if len(sizes) != N or len(flips) != N:
+            raise ValueError("one output size and one flip flag per image")
+        for im in imgs:
+            if im.dim() != 3 or im.shape[2] != 3 or im.dtype != torch.uint8:
+                raise ValueError("images must be (H, W, 3) uint8 (a CHW image as x.permute(1, 2, 0))")
+        arr = (ResizeImage * N)()
+        self.offsets, total, max_k = [], 0, 0
+        with torch.cuda.device(dev):
+            for n, (im, (h, w)) in enumerate(zip(imgs, sizes)):
+                H, W = int(im.shape[0]), int(im.shape[1])
+                if H <= 0 or W <= 0 or h <= 0 or w <= 0:
+                    raise ValueError("image and output sizes must be positive")
+                if H > 4 * h or W > 4 * w:
+                    raise ValueError(f"resize {H}x{W} -> {h}x{w}: down-scales beyond 4 per axis are not supported")
+                if h * w > 0x7FFFFFFF:
+                    raise ValueError("output plane too large")
+                kxo, kxs = _resize_table(dev, W, w)
+                kyo, kys = _resize_table(dev, H, h)
+                max_k = max(max_k, kxs, kys)
+                r = arr[n]
+                r.src = im.data_ptr()
+                r.stride_row, r.stride_px, r.stride_ch = (int(v) for v in im.stride())
+                r.in_h, r.in_w, r.out_h, r.out_w = H, W, h, w
+                r.out_offset = total
+                r.hflip = int(flips[n])
+                r.kx_offset, r.kx_size, r.ky_offset, r.ky_size = kxo, kxs, kyo, kys
+                self.offsets.append(total)
+                total += 3 * h * w
+            self.records = _struct_array_to_device(arr, dev)
+            self.coeffs = _resize_arena[dev.index if dev.index is not None else torch.cuda.current_device()]["buf"]
+        self.images, self.dev, self.n, self.sizes, self.nbytes, self.max_k = imgs, dev, N, sizes, total, max_k
+
+    def launch(self, out: Tensor) -> None:
+        if out.device != self.dev or out.dtype != torch.uint8 or out.numel() < self.nbytes or not out.is_contiguous():
+            raise ValueError("out must be a contiguous uint8 tensor of at least nbytes on the images' device")
+        with torch.cuda.device(self.dev):
+            check(_lib.lib().sfod_resize_pil(self.records.data_ptr(), self.n, self.coeffs.data_ptr(), out.data_ptr(),
+                                             max(h for h, _ in self.sizes), max(w for _, w in self.sizes), self.max_k,
+                                             _stream(self.dev)), "sfod_resize_pil")
+
+
+def resize_pil(images: Union[Tensor, Sequence[Tensor]], sizes: Sequence[Tuple[int, int]],
+               hflip: Optional[Sequence[bool]] = None) -> Union[Tensor, List[Tensor]]:
+    """``np.flip(np.asarray(Image.fromarray(img).resize((w, h), Image.BILINEAR)), 1)`` (flip optional) for every image of a batch,
+    bit for bit, transposed to CHW -- detectron2's ResizeTransform (uint8 path) + HFlipTransform + the mapper's HWC -> CHW copy.
+
+    ``images``: a (N, H, W, 3) tensor, or a list of (H, W, 3) CUDA uint8 tensors or views of any strides (a CHW image passes as
+    ``x.permute(1, 2, 0)``); ``sizes[n]`` = output (h, w); ``hflip[n]`` = mirror the output horizontally.  Returns a (N, 3, h, w)
+    tensor when all output sizes are equal, otherwise a list of (3, h, w) views into one allocation.  One launch."""
+    with _timed("resize_pil"):
+        plan = ResizePlan(images, sizes, hflip)
+        out = torch.empty(plan.nbytes, dtype=torch.uint8, device=plan.dev)
+        plan.launch(out)
+    N, sz = plan.n, plan.sizes
+    if all(s == sz[0] for s in sz):
+        return out.view(N, 3, sz[0][0], sz[0][1])
+    return [out[o:o + 3 * h * w].view(3, h, w) for o, (h, w) in zip(plan.offsets, sz)]
