@@ -46,7 +46,8 @@ enum sfod_status {
 enum sfod_layout { SFOD_NCHW = 0, SFOD_NHWC = 1 };
 enum sfod_dtype { SFOD_F32 = 0, SFOD_I64 = 1, SFOD_U8 = 2 };
 
-/* Changes whenever an entry point keeps its name but changes its arguments; a binding refuses a library of another version. */
+/* Changes whenever an entry point keeps its name but changes its arguments, or a parameter record field changes its meaning;
+ * a binding refuses a library of another version. */
 int sfod_abi_version(void);
 /* sizeof() of the parameter structs as this library was compiled (which: 0 sfod_ema_tensor, 1 sfod_rpn_params,
  * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params, 6 sfod_resize_image; 0 for anything else) -- lets a foreign
@@ -103,8 +104,6 @@ int sfod_roi_pool_fwd(const float *input, const float *rois, int N, int C, int H
                       float spatial_scale, float *output, int32_t *argmax, sfod_stream_t stream);
 int sfod_roi_pool_bwd(const float *grad_out, const float *rois, const int32_t *argmax, int N, int C, int H, int W,
                       int R, int PH, int PW, float *grad_in, sfod_stream_t stream);
-/* layout helper used by the wrappers (tiled shared-memory transpose) */
-int sfod_nchw_to_nhwc(const float *src, float *dst, int N, int C, int HW, sfod_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * NMS with torchvision semantics.  Replaces torchvision.ops.nms / batched_nms as reached
@@ -369,29 +368,20 @@ int sfod_p2p_status(const sfod_p2p_comm_t *comm, uint64_t *exchanges, uint32_t *
  * daod/data/mappers/two_crop_augmentation_mapper.py:141-157: RandomApply(ColorJitter(0.4, 0.4, 0.4, 0.1), 0.8),
  * RandomGrayscale(0.2), RandomApply(GaussianBlur((0.1, 2.0)), 0.5), 3 x RandomErasing(value="random").
  * Images are (N, 3, H, W) uint8, RGB planes.  The random decisions are drawn by the caller (as torchvision draws them) and
- * passed as per-image parameter records in DEVICE memory. */
+ * passed as per-image parameter records in DEVICE memory.  The pixel arithmetic is Pillow's, bit for bit: the reference's mapper
+ * hands PIL images to the transforms, so torchvision's PIL path is what it executes. */
 typedef struct sfod_jitter_params {
   int32_t n_ops;          /* 0 = ColorJitter not applied; else 4 */
   int32_t op[4];          /* order of application: 0 brightness, 1 contrast, 2 saturation, 3 hue */
-  float factor[4];        /* factor of op[k] */
-  float one_minus[4];     /* (float)(1.0 - factor) computed in double (what torchvision's _blend multiplies img2 with) */
+  float factor[4];        /* blend alpha of op[k] (brightness / contrast / saturation) */
+  int32_t hue_shift[4];   /* hue op: the shift byte uint8(int32(255 * hue)); ignored for the other ops */
   int32_t grayscale;      /* != 0: RandomGrayscale hit (3-channel gray after the jitter) */
 } sfod_jitter_params;
-/* uint8 tensor arithmetic of torchvision.transforms.functional (adjust_brightness / contrast / saturation / hue,
- * rgb_to_grayscale), operation by operation.  workspace: N * 8 bytes.  out may alias images. */
-int sfod_color_jitter(const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
-                      size_t workspace_bytes, uint8_t *out, sfod_stream_t stream);
-/* The same ops in PILLOW's arithmetic -- what the reference executes, because its data mapper hands PIL images to the transforms
- * (daod/data/mappers/two_crop_augmentation_mapper.py:141-157): Image.blend against a black / mean-gray / gray degenerate image
- * (ImageEnhance.Brightness / Contrast / Color), convert("L") = (19595 R + 38470 G + 7471 B + 0x8000) >> 16, adjust_hue through
- * convert("HSV") with the shift byte uint8(int32(255 * hue)).  Same record layout; for a hue op `one_minus[k]` carries the shift byte
- * (as a float), `factor[k]` is the blend alpha of the other ops.  Bit-exact against torchvision's PIL path (tests). */
+/* ColorJitter + RandomGrayscale: Image.blend against a black / mean-gray / gray degenerate image (ImageEnhance.Brightness /
+ * Contrast / Color), convert("L") = (19595 R + 38470 G + 7471 B + 0x8000) >> 16, adjust_hue through convert("HSV").
+ * Bit-exact against torchvision's PIL path (tests).  workspace: N * 8 bytes.  out may alias images. */
 int sfod_color_jitter_pil(const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
                           size_t workspace_bytes, uint8_t *out, sfod_stream_t stream);
-/* Separable Gaussian blur with reflect padding and round-half-even to uint8.  taps_dev: (N, 31) floats, image n uses
- * taps[n][0 .. 2*radius[n]]; radius_dev[n] = 0 copies the image (RandomApply miss); max_radius = max over n (<= 15). */
-int sfod_gaussian_blur(const uint8_t *images, int N, int H, int W, const float *taps_dev, const int32_t *radius_dev,
-                       int max_radius, uint8_t *out, sfod_stream_t stream);
 /* Pillow's ImageFilter.GaussianBlur bit for bit -- the filter the reference actually applies (reference
  * daod/data/transforms/augmentations.py:18-21): three extended-box-blur passes per axis in 8.24 fixed point, each rounded to
  * uint8, edges replicated (Pillow src/libImaging/BoxBlur.c).  Per image: radius_dev[n] = integer box radius (-1: copy the image,

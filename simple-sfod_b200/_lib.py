@@ -25,7 +25,7 @@ class EmaTensor(C.Structure):
 
 
 class JitterParams(C.Structure):
-    _fields_ = [("n_ops", C.c_int32), ("op", C.c_int32 * 4), ("factor", C.c_float * 4), ("one_minus", C.c_float * 4), ("grayscale", C.c_int32)]
+    _fields_ = [("n_ops", C.c_int32), ("op", C.c_int32 * 4), ("factor", C.c_float * 4), ("hue_shift", C.c_int32 * 4), ("grayscale", C.c_int32)]
 
 
 class EraseParams(C.Structure):
@@ -62,7 +62,7 @@ class P2PComm(C.Structure):
 
 
 # sfod_abi_version() of the library this binding is written for, and the struct mirrors in the order of sfod_abi_sizeof(which)
-ABI_VERSION = 2
+ABI_VERSION = 3
 ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams, ResizeImage)
 
 
@@ -84,7 +84,6 @@ SIGNATURES = {
                                      C.c_size_t, c_ptr]),
     "sfod_roi_pool_fwd": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 7 + [C.c_float, c_ptr, c_ptr, c_ptr]),
     "sfod_roi_pool_bwd": (C.c_int, [c_ptr, c_ptr, c_ptr] + [C.c_int] * 7 + [c_ptr, c_ptr]),
-    "sfod_nchw_to_nhwc": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
     "sfod_nms_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "sfod_nms": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int64, C.c_double, C.c_int64, c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "sfod_rpn_select_workspace_bytes": (C.c_size_t, [C.POINTER(RpnParams)]),
@@ -101,9 +100,7 @@ SIGNATURES = {
     "sfod_iou_match_workspace_bytes": (C.c_size_t, [C.c_int]),
     "sfod_iou_match": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_int), C.c_int, C.c_int,
                                  c_ptr, c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
-    "sfod_color_jitter": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_size_t, c_ptr, c_ptr]),
     "sfod_color_jitter_pil": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_size_t, c_ptr, c_ptr]),
-    "sfod_gaussian_blur": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "sfod_gaussian_blur_pil": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "sfod_random_erase": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_uint64, c_ptr]),
     "sfod_resize_pil": (C.c_int, [c_ptr, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),

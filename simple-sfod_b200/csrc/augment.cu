@@ -8,16 +8,10 @@
 // records; the kernels do the pixel work.
 //
 // Arithmetic contract (this TU is compiled with -fmad=false; every op is separately rounded):
-//   * brightness / contrast / saturation / hue / grayscale follow torchvision.transforms.functional on uint8 TENSORS
-//     (torchvision/transforms/_functional_tensor.py: rgb_to_grayscale :148-168, _blend :258-261, _rgb2hsv :264-300,
-//     _hsv2rgb :303-321, adjust_hue :196-221) operation by operation -- bit-exact, except that the image mean of the contrast
-//     op is the exact integer sum / n here and a float32 cascade sum in ATen (differs in the last ulp: a pixel can move by one
-//     level when its blend lands within 1e-5 of an integer);
-//   * ... and, by default, the SAME ops in Pillow's arithmetic (jitter_pixel<true>): the reference's mapper hands PIL images to the
-//     transforms, so torchvision's PIL path (ImageEnhance / Image.convert) is what the reference executes -- bit-exact;
+//   * brightness / contrast / saturation / hue / grayscale follow Pillow's arithmetic (jitter_pixel): the reference's mapper hands
+//     PIL images to the transforms, so torchvision's PIL path (ImageEnhance / Image.convert) is what the reference executes -- bit-exact;
 //   * Gaussian blur: pil_blur_kernel reproduces Pillow's ImageFilter.GaussianBlur (three extended-box passes per axis in 8.24
-//     fixed point) bit for bit -- the reference's filter; gauss_blur_kernel is a true separable Gaussian with torchvision's taps,
-//     reflect padding, round-half-to-even to uint8 (optional);
+//     fixed point) bit for bit -- the reference's filter;
 //   * erasing writes byte(255 * v) (v ~ N(0, 1) from a counter-based generator, or a caller-provided noise tensor) into the
 //     rectangles, which is what ToTensor -> erase(value="random") -> ToPILImage (`pic.mul(255).byte()`) leaves there.
 #include "common.cuh"
@@ -30,68 +24,15 @@ constexpr int kOpBrightness = 0, kOpContrast = 1, kOpSaturation = 2, kOpHue = 3;
 struct JitterRec {     // one per image; mirrors sfod_jitter_params
   int n_ops;           // 0..4 (0: ColorJitter not applied)
   int op[4];           // application order (torchvision: a random permutation of 0..3)
-  float factor[4];     // factor of op[k] (float32 of the Python float)
-  float one_minus[4];  // float32 of (1.0 - factor) evaluated in double, as Python does before the tensor op sees it
+  float factor[4];     // blend alpha of op[k] (float32 of the Python float)
+  int hue_shift[4];    // hue op: the shift byte uint8(int32(255 * hue)); ignored for the other ops
   int grayscale;       // RandomGrayscale hit: 3-channel gray AFTER the jitter
 };
 
-__device__ __forceinline__ float u8f(unsigned char v) { return (float)v; }
-__device__ __forceinline__ unsigned char trunc_u8(float v) { return (unsigned char)(int)fminf(fmaxf(v, 0.0f), 255.0f); }
-
-// torchvision rgb_to_grayscale on uint8: (0.2989 r + 0.587 g + 0.114 b).to(uint8)
-__device__ __forceinline__ unsigned char gray_u8(unsigned char r, unsigned char g, unsigned char b) {
-  const float l = __fadd_rn(__fadd_rn(__fmul_rn(0.2989f, u8f(r)), __fmul_rn(0.587f, u8f(g))), __fmul_rn(0.114f, u8f(b)));
-  return (unsigned char)(int)l;
-}
-// _blend(img1, img2, ratio) for uint8 img1: (ratio * img1 + (1 - ratio) * img2).clamp(0, 255).to(uint8)
-__device__ __forceinline__ unsigned char blend_u8(unsigned char a, float other, float ratio, float one_minus) {
-  return trunc_u8(__fadd_rn(__fmul_rn(ratio, u8f(a)), __fmul_rn(one_minus, other)));
-}
-
-__device__ __forceinline__ void hue_shift(unsigned char &R, unsigned char &G, unsigned char &B, float hue) {
-  const float r = __fdiv_rn(u8f(R), 255.0f), g = __fdiv_rn(u8f(G), 255.0f), b = __fdiv_rn(u8f(B), 255.0f);
-  const float maxc = fmaxf(fmaxf(r, g), b), minc = fminf(fminf(r, g), b);
-  const bool eqc = maxc == minc;
-  const float cr = __fsub_rn(maxc, minc);
-  const float s = __fdiv_rn(cr, eqc ? 1.0f : maxc);
-  const float div = eqc ? 1.0f : cr;
-  const float rc = __fdiv_rn(__fsub_rn(maxc, r), div), gc = __fdiv_rn(__fsub_rn(maxc, g), div), bc = __fdiv_rn(__fsub_rn(maxc, b), div);
-  const float hr = (maxc == r) ? __fsub_rn(bc, gc) : 0.0f;
-  const float hg = ((maxc == g) && (maxc != r)) ? __fsub_rn(__fadd_rn(2.0f, rc), bc) : 0.0f;
-  const float hb = ((maxc != g) && (maxc != r)) ? __fsub_rn(__fadd_rn(4.0f, gc), rc) : 0.0f;
-  float h = __fadd_rn(__fadd_rn(hr, hg), hb);
-  h = fmodf(__fadd_rn(__fdiv_rn(h, 6.0f), 1.0f), 1.0f);
-  // h = (h + hue_factor) % 1.0  (torch.remainder: result has the sign of the divisor)
-  h = __fadd_rn(h, hue);
-  h = __fsub_rn(h, floorf(h));           // remainder(h, 1) for |h| < 2: h - floor(h) is exact in this range
-  if (h >= 1.0f) h = 0.0f;               // -tiny + 1 rounds to 1.0: remainder returns a value in [0, 1)
-  const float v = maxc;
-  const float h6 = __fmul_rn(h, 6.0f);
-  const float fi = floorf(h6);
-  const float f = __fsub_rn(h6, fi);
-  int i = (int)fi; i = i % 6;
-  const float p = fminf(fmaxf(__fmul_rn(v, __fsub_rn(1.0f, s)), 0.0f), 1.0f);
-  const float q = fminf(fmaxf(__fmul_rn(v, __fsub_rn(1.0f, __fmul_rn(s, f))), 0.0f), 1.0f);
-  const float t = fminf(fmaxf(__fmul_rn(v, __fsub_rn(1.0f, __fmul_rn(s, __fsub_rn(1.0f, f)))), 0.0f), 1.0f);
-  float ro, go, bo;
-  switch (i) {
-    case 0: ro = v; go = t; bo = p; break;
-    case 1: ro = q; go = v; bo = p; break;
-    case 2: ro = p; go = v; bo = t; break;
-    case 3: ro = p; go = q; bo = v; break;
-    case 4: ro = t; go = p; bo = v; break;
-    default: ro = v; go = p; bo = q; break;
-  }
-  // convert_image_dtype(float -> uint8): image.mul(255 + 1.0 - 1e-3).to(uint8)
-  R = (unsigned char)(int)__fmul_rn(ro, 255.999f);
-  G = (unsigned char)(int)__fmul_rn(go, 255.999f);
-  B = (unsigned char)(int)__fmul_rn(bo, 255.999f);
-}
-
-// ---- the same ops in PILLOW's arithmetic: the reference hands PIL images to torchvision's transforms
-// (daod/data/mappers/two_crop_augmentation_mapper.py:141-157), whose PIL path is ImageEnhance / Image.convert, not the tensor
-// code above.  Restated from Pillow's libImaging (Blend.c, Convert.c) and torchvision/transforms/_functional_pil.py and pinned
-// against the installed Pillow (oracle/pil_cpu.py, tests): bit-exact.
+// ---- ColorJitter / RandomGrayscale in PILLOW's arithmetic: the reference hands PIL images to torchvision's transforms
+// (daod/data/mappers/two_crop_augmentation_mapper.py:141-157), whose PIL path is ImageEnhance / Image.convert.  Restated from
+// Pillow's libImaging (Blend.c, Convert.c) and torchvision/transforms/_functional_pil.py and pinned against the installed Pillow
+// (oracle/pil_cpu.py, tests): bit-exact.
 //   convert("L"):   L = (19595 R + 38470 G + 7471 B + 0x8000) >> 16
 //   Image.blend(degenerate, image, alpha): (UINT8)(float)(deg + alpha * (img - deg)), clipped to [0, 255] when alpha is outside [0, 1]
 //   Brightness: degenerate = 0;  Contrast: degenerate = int(mean(L) + 0.5);  Color (saturation): degenerate = L
@@ -147,29 +88,15 @@ __device__ __forceinline__ void pil_hue_shift(unsigned char &R, unsigned char &G
   R = (unsigned char)ro; G = (unsigned char)go; B = (unsigned char)bo;
 }
 
-template <bool kPil>
-__device__ __forceinline__ unsigned char gray_of(unsigned char r, unsigned char g, unsigned char b) { return kPil ? pil_L(r, g, b) : gray_u8(r, g, b); }
-
-// applies ops [0, upto) of the record to one pixel; `mean` = gray mean of the image at the point where contrast is applied
-// (kPil: the integer int(mean + 0.5); the hue record carries the shift byte in one_minus)
-template <bool kPil>
-__device__ __forceinline__ void jitter_pixel(const JitterRec &p, int upto, float mean, unsigned char &r, unsigned char &g, unsigned char &b) {
+// applies ops [0, upto) of the record to one pixel; `mean` = int(mean(L) + 0.5) of the image at the point where contrast is applied
+__device__ __forceinline__ void jitter_pixel(const JitterRec &p, int upto, int mean, unsigned char &r, unsigned char &g, unsigned char &b) {
   for (int k = 0; k < upto; ++k) {
-    const float f = p.factor[k], om = p.one_minus[k];
-    if (kPil) {
-      switch (p.op[k]) {
-        case kOpBrightness: r = pil_blend(0, r, f); g = pil_blend(0, g, f); b = pil_blend(0, b, f); break;
-        case kOpContrast: { const int m = (int)mean; r = pil_blend(m, r, f); g = pil_blend(m, g, f); b = pil_blend(m, b, f); break; }
-        case kOpSaturation: { const int l = pil_L(r, g, b); r = pil_blend(l, r, f); g = pil_blend(l, g, f); b = pil_blend(l, b, f); break; }
-        default: pil_hue_shift(r, g, b, (int)om); break;
-      }
-    } else {
-      switch (p.op[k]) {
-        case kOpBrightness: r = blend_u8(r, 0.0f, f, om); g = blend_u8(g, 0.0f, f, om); b = blend_u8(b, 0.0f, f, om); break;
-        case kOpContrast: r = blend_u8(r, mean, f, om); g = blend_u8(g, mean, f, om); b = blend_u8(b, mean, f, om); break;
-        case kOpSaturation: { const float l = u8f(gray_u8(r, g, b)); r = blend_u8(r, l, f, om); g = blend_u8(g, l, f, om); b = blend_u8(b, l, f, om); break; }
-        default: hue_shift(r, g, b, f); break;
-      }
+    const float f = p.factor[k];
+    switch (p.op[k]) {
+      case kOpBrightness: r = pil_blend(0, r, f); g = pil_blend(0, g, f); b = pil_blend(0, b, f); break;
+      case kOpContrast: r = pil_blend(mean, r, f); g = pil_blend(mean, g, f); b = pil_blend(mean, b, f); break;
+      case kOpSaturation: { const int l = pil_L(r, g, b); r = pil_blend(l, r, f); g = pil_blend(l, g, f); b = pil_blend(l, b, f); break; }
+      default: pil_hue_shift(r, g, b, p.hue_shift[k]); break;
     }
   }
 }
@@ -180,7 +107,6 @@ __device__ __forceinline__ int contrast_pos(const JitterRec &p) {
 }
 
 // pass A: sum of the gray levels of every image at the point where its contrast op applies (exact integer sum)
-template <bool kPil>
 __global__ void __launch_bounds__(kJThreads) jitter_gray_sum_kernel(const unsigned char *__restrict__ img, const JitterRec *__restrict__ recs,
                                                                     int HW, unsigned long long *__restrict__ sums) {
   const int n = blockIdx.y;
@@ -191,87 +117,28 @@ __global__ void __launch_bounds__(kJThreads) jitter_gray_sum_kernel(const unsign
   unsigned int local = 0;
   for (int i = blockIdx.x * kJThreads + threadIdx.x; i < HW; i += gridDim.x * kJThreads) {
     unsigned char r = R[i], g = G[i], b = B[i];
-    jitter_pixel<kPil>(p, cp, 0.0f, r, g, b);
-    local += gray_of<kPil>(r, g, b);
+    jitter_pixel(p, cp, 0, r, g, b);
+    local += pil_L(r, g, b);
   }
   local = __reduce_add_sync(0xFFFFFFFFu, local);
   if ((threadIdx.x & 31) == 0 && local) atomicAdd(sums + n, (unsigned long long)local);
 }
 
 // pass B: the whole op sequence (+ RandomGrayscale) per pixel
-template <bool kPil>
 __global__ void __launch_bounds__(kJThreads) jitter_apply_kernel(const unsigned char *__restrict__ img, const JitterRec *__restrict__ recs,
                                                                  const unsigned long long *__restrict__ sums, int HW,
                                                                  unsigned char *__restrict__ out) {
   const int n = blockIdx.y;
   const JitterRec p = recs[n];
-  // torch.mean of the float32 gray image; here: exact sum / n rounded once
-  // (kPil: ImageStat mean = sum / count as a Python float, then int(mean + 0.5))
-  const double dmean = contrast_pos(p) >= 0 ? (double)sums[n] / (double)HW : 0.0;
-  const float mean = kPil ? (float)(int)(dmean + 0.5) : (float)dmean;
+  // ImageStat mean = sum / count as a Python float, then int(mean + 0.5)
+  const int mean = contrast_pos(p) >= 0 ? (int)((double)sums[n] / (double)HW + 0.5) : 0;
   const unsigned char *R = img + (size_t)n * 3 * HW, *G = R + HW, *B = G + HW;
   unsigned char *Ro = out + (size_t)n * 3 * HW, *Go = Ro + HW, *Bo = Go + HW;
   for (int i = blockIdx.x * kJThreads + threadIdx.x; i < HW; i += gridDim.x * kJThreads) {
     unsigned char r = R[i], g = G[i], b = B[i];
-    jitter_pixel<kPil>(p, p.n_ops, mean, r, g, b);
-    if (p.grayscale) { const unsigned char l = gray_of<kPil>(r, g, b); r = g = b = l; }
+    jitter_pixel(p, p.n_ops, mean, r, g, b);
+    if (p.grayscale) { const unsigned char l = pil_L(r, g, b); r = g = b = l; }
     Ro[i] = r; Go[i] = g; Bo[i] = b;
-  }
-}
-
-// ---- Gaussian blur: one CTA = 32 x 32 output pixels of one plane; (32 + 2R)^2 input tile in shared memory (reflect padding),
-// horizontal then vertical pass in fp32, round-half-to-even (torch.round) to uint8.  taps: (N, 2*kMaxRadius+1) floats, radius: (N).
-constexpr int kMaxRadius = 15;
-constexpr int kTile = 32;
-
-__device__ __forceinline__ int reflect(int i, int n) {   // torch 'reflect' padding (no edge repeat); valid for pad < n
-  if (i < 0) i = -i;
-  if (i >= n) i = 2 * (n - 1) - i;
-  return i;
-}
-
-__global__ void __launch_bounds__(256) gauss_blur_kernel(const unsigned char *__restrict__ img, const float *__restrict__ taps,
-                                                         const int *__restrict__ radius, int H, int W, unsigned char *__restrict__ out) {
-  extern __shared__ float gb_smem[];
-  const int plane = blockIdx.z;          // n * 3 + c
-  const int n = plane / 3;
-  const int Rr = radius[n];
-  const unsigned char *src = img + (size_t)plane * H * W;
-  unsigned char *dst = out + (size_t)plane * H * W;
-  const int x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile;
-  if (Rr <= 0) {                          // not blurred: copy
-    for (int t = threadIdx.x; t < kTile * kTile; t += 256) {
-      const int y = y0 + t / kTile, x = x0 + t % kTile;
-      if (y < H && x < W) dst[(size_t)y * W + x] = src[(size_t)y * W + x];
-    }
-    return;
-  }
-  const int TW = kTile + 2 * Rr;
-  float *tile = gb_smem;                  // TW x TW input
-  float *hbuf = gb_smem + TW * TW;        // TW rows x kTile columns (horizontal pass)
-  float *w = hbuf + TW * kTile;           // 2R + 1 taps
-  const float *tp = taps + (size_t)n * (2 * kMaxRadius + 1);
-  for (int t = threadIdx.x; t < 2 * Rr + 1; t += 256) w[t] = tp[t];
-  for (int t = threadIdx.x; t < TW * TW; t += 256) {
-    const int ty = t / TW, tx = t - ty * TW;
-    const int y = reflect(y0 + ty - Rr, H), x = reflect(x0 + tx - Rr, W);
-    tile[t] = (float)src[(size_t)y * W + x];
-  }
-  __syncthreads();
-  for (int t = threadIdx.x; t < TW * kTile; t += 256) {
-    const int ty = t / kTile, tx = t - ty * kTile;
-    float acc = 0.0f;
-    for (int k = 0; k <= 2 * Rr; ++k) acc = __fadd_rn(acc, __fmul_rn(w[k], tile[ty * TW + tx + k]));
-    hbuf[t] = acc;
-  }
-  __syncthreads();
-  for (int t = threadIdx.x; t < kTile * kTile; t += 256) {
-    const int ty = t / kTile, tx = t - ty * kTile;
-    const int y = y0 + ty, x = x0 + tx;
-    if (y >= H || x >= W) continue;
-    float acc = 0.0f;
-    for (int k = 0; k <= 2 * Rr; ++k) acc = __fadd_rn(acc, __fmul_rn(w[k], hbuf[(ty + k) * kTile + tx]));
-    dst[(size_t)y * W + x] = (unsigned char)(int)fminf(fmaxf(rintf(acc), 0.0f), 255.0f);
   }
 }
 
@@ -283,6 +150,7 @@ __global__ void __launch_bounds__(256) gauss_blur_kernel(const unsigned char *__
 // ops.pil_blur_params).  All six passes run on one shared-memory tile: 32 x 32 outputs plus a halo of 3 (r + 1) pixels per side;
 // every pass clamps in IMAGE coordinates, exactly as the line-by-line C code does, so borders are identical too.
 constexpr int kPilMaxRadius = 9;   // box radius; sigma <= ~10
+constexpr int kTile = 32;
 
 __global__ void __launch_bounds__(256) pil_blur_kernel(const unsigned char *__restrict__ img, const int *__restrict__ radius,
                                                        const unsigned *__restrict__ wws, const unsigned *__restrict__ fws, int H, int W,
@@ -394,8 +262,8 @@ __global__ void __launch_bounds__(256) erase_kernel(unsigned char *__restrict__ 
 }  // namespace
 
 // =========================================================================== C ABI
-static int color_jitter_impl(bool pil, const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
-                             size_t workspace_bytes, uint8_t *out, sfod_stream_t stream) {
+SFOD_API int sfod_color_jitter_pil(const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
+                                   size_t workspace_bytes, uint8_t *out, sfod_stream_t stream) {
   static_assert(sizeof(sfod_jitter_params) == sizeof(JitterRec), "parameter record layout");
   if (N < 0 || H <= 0 || W <= 0) return SFOD_ERR_INVALID_ARG;
   if (N == 0) return SFOD_OK;
@@ -407,36 +275,9 @@ static int color_jitter_impl(bool pil, const uint8_t *images, int N, int H, int 
   const int HW = H * W;
   const unsigned gx = (unsigned)min(SFOD_NUM_SMS * 2, (HW + kJThreads - 1) / kJThreads);
   const JitterRec *recs = reinterpret_cast<const JitterRec *>(params_dev);
-  if (pil) jitter_gray_sum_kernel<true><<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, HW, sums);
-  else jitter_gray_sum_kernel<false><<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, HW, sums);
+  jitter_gray_sum_kernel<<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, HW, sums);
   SFOD_LAUNCH_CHECK();
-  if (pil) jitter_apply_kernel<true><<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, sums, HW, out);
-  else jitter_apply_kernel<false><<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, sums, HW, out);
-  SFOD_LAUNCH_CHECK();
-  return SFOD_OK;
-}
-
-SFOD_API int sfod_color_jitter(const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
-                               size_t workspace_bytes, uint8_t *out, sfod_stream_t stream) {
-  return color_jitter_impl(false, images, N, H, W, params_dev, workspace, workspace_bytes, out, stream);
-}
-
-SFOD_API int sfod_color_jitter_pil(const uint8_t *images, int N, int H, int W, const sfod_jitter_params *params_dev, void *workspace,
-                                   size_t workspace_bytes, uint8_t *out, sfod_stream_t stream) {
-  return color_jitter_impl(true, images, N, H, W, params_dev, workspace, workspace_bytes, out, stream);
-}
-
-SFOD_API int sfod_gaussian_blur(const uint8_t *images, int N, int H, int W, const float *taps_dev, const int32_t *radius_dev,
-                                int max_radius, uint8_t *out, sfod_stream_t stream) {
-  if (N < 0 || H <= 0 || W <= 0 || max_radius < 0 || max_radius > kMaxRadius) return SFOD_ERR_INVALID_ARG;
-  if (max_radius >= H || max_radius >= W) return SFOD_ERR_INVALID_ARG;   // reflect padding needs pad < size
-  if (N == 0) return SFOD_OK;
-  if (!images || !taps_dev || !radius_dev || !out || images == out) return SFOD_ERR_INVALID_ARG;
-  const int TW = kTile + 2 * max_radius;
-  const size_t smem = ((size_t)TW * TW + (size_t)TW * kTile + 2 * kMaxRadius + 1) * sizeof(float);
-  SFOD_CUDA_TRY(cudaFuncSetAttribute(gauss_blur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  dim3 grid((W + kTile - 1) / kTile, (H + kTile - 1) / kTile, N * 3);
-  gauss_blur_kernel<<<grid, 256, smem, sfod_cu(stream)>>>(images, taps_dev, radius_dev, H, W, out);
+  jitter_apply_kernel<<<dim3(gx, N), kJThreads, 0, st>>>(images, recs, sums, HW, out);
   SFOD_LAUNCH_CHECK();
   return SFOD_OK;
 }

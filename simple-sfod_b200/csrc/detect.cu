@@ -415,7 +415,7 @@ SFOD_API int sfod_class_histogram(const float *values, const int64_t *classes, c
   return SFOD_OK;
 }
 
-SFOD_API int sfod_abi_version(void) { return 2; }
+SFOD_API int sfod_abi_version(void) { return 3; }
 
 SFOD_API size_t sfod_abi_sizeof(int which) {
   switch (which) {

@@ -1121,11 +1121,6 @@ bool sep_supported(int C, int H, int W, int PH, int PW) {
 }  // namespace
 
 // =========================================================================== C ABI
-SFOD_API int sfod_nchw_to_nhwc(const float *src, float *dst, int N, int C, int HW, sfod_stream_t stream) {
-  if (!src || !dst) return SFOD_ERR_INVALID_ARG;
-  return launch_transpose(src, dst, N, C, HW, sfod_cu(stream));
-}
-
 SFOD_API size_t sfod_roi_align_fwd_workspace_bytes(int N, int C, int H, int W, int R, int layout, int exact) {
   // exact kernel reads NCHW, separable kernel reads NHWC: a converted copy is needed when layouts differ; the separable
   // kernel also needs one table record per ROI and its work counter

@@ -83,24 +83,19 @@ def draw_params(N: int, H: int, W: int, generator: Optional[torch.Generator] = N
 
 
 def strong_augment(images: Tensor, params: Optional[List[Dict]] = None, generator: Optional[torch.Generator] = None,
-                   noise: Optional[Tensor] = None, seed: Optional[int] = None, blur: str = "pil", arithmetic: str = "pil") -> Tensor:
+                   noise: Optional[Tensor] = None, seed: Optional[int] = None) -> Tensor:
     """(N, 3, H, W) uint8 RGB CUDA batch -> strongly augmented uint8 batch (a new tensor).
 
-    ``arithmetic="pil"`` (default): ColorJitter / RandomGrayscale in Pillow's arithmetic (torchvision's PIL path, which the
-    reference's mapper takes: daod/data/mappers/two_crop_augmentation_mapper.py:141-157), bit for bit; ``"tensor"``: torchvision's
-    uint8-tensor arithmetic.
-
-    ``blur="pil"`` (default) is the reference's filter, ``PIL.ImageFilter.GaussianBlur(radius=sigma)`` (reference
-    daod/data/transforms/augmentations.py:18-21) reproduced bit for bit (``ops.gaussian_blur_pil``: Pillow's three extended
-    box-blur passes per axis); ``blur="gaussian"`` is a true Gaussian convolution with torchvision's taps (``ops.gaussian_blur``)."""
-    if blur not in ("pil", "gaussian"):
-        raise ValueError("blur must be 'pil' or 'gaussian'")
+    ColorJitter / RandomGrayscale run in Pillow's arithmetic (torchvision's PIL path, which the reference's mapper takes:
+    daod/data/mappers/two_crop_augmentation_mapper.py:141-157), bit for bit.  The blur is the reference's filter,
+    ``PIL.ImageFilter.GaussianBlur(radius=sigma)`` (reference daod/data/transforms/augmentations.py:18-21) reproduced bit for bit
+    (``ops.gaussian_blur_pil``: Pillow's three extended box-blur passes per axis)."""
     N, _, H, W = images.shape
     if params is None:
         params = draw_params(N, H, W, generator)
-    x = ops.color_jitter(images, params, arithmetic=arithmetic)
+    x = ops.color_jitter(images, params)
     if any(p["sigma"] is not None for p in params):
-        x = (ops.gaussian_blur_pil if blur == "pil" else ops.gaussian_blur)(x, [p["sigma"] for p in params])
+        x = ops.gaussian_blur_pil(x, [p["sigma"] for p in params])
     if any(p["rects"] for p in params):
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,), generator=generator if generator is not None else torch.default_generator))

@@ -284,17 +284,6 @@ def roi_pool(input: Tensor, boxes: Union[Tensor, List[Tensor]], output_size, spa
     return _RoIPoolFn.apply(input, rois, ph, pw, spatial_scale)
 
 
-def nchw_to_nhwc(x: Tensor) -> Tensor:
-    """Returns a channels_last tensor with x's values (our transpose kernel, not a torch copy)."""
-    dev = _require_cuda(x)
-    xin = _f32c(x)
-    N, Cc, H, W = xin.shape
-    out = torch.empty((N, Cc, H, W), dtype=torch.float32, device=dev, memory_format=torch.channels_last)
-    with torch.cuda.device(dev):
-        check(_lib.lib().sfod_nchw_to_nhwc(xin.data_ptr(), out.data_ptr(), N, Cc, H * W, _stream(dev)), "sfod_nchw_to_nhwc")
-    return out
-
-
 # ----------------------------------------------------------------------------------------------- box coder / softmax
 def apply_deltas(deltas: Tensor, boxes: Tensor, weights: Sequence[float], scale_clamp: float = SCALE_CLAMP) -> Tensor:
     """detectron2 Box2BoxTransform.apply_deltas: deltas (R, 4k), boxes (R, 4) -> (R, 4k)."""
@@ -817,15 +806,11 @@ def _struct_array_to_device(arr, dev: torch.device) -> Tensor:
     return torch.frombuffer(bytearray(raw), dtype=torch.uint8).to(dev)
 
 
-def color_jitter(images: Tensor, params: Sequence[dict], arithmetic: str = "tensor") -> Tensor:
+def color_jitter(images: Tensor, params: Sequence[dict]) -> Tensor:
     """torchvision ColorJitter (+ RandomGrayscale) on a uint8 batch with per-image decisions ``params[n] = dict(order=[...],
     factors=[...], grayscale=bool)``: ``order`` lists op codes (0 brightness, 1 contrast, 2 saturation, 3 hue) in application
-    order with their ``factors`` (Python floats); an empty order = jitter not applied.  ``arithmetic="tensor"`` follows
-    torchvision's uint8-tensor code, ``"pil"`` follows its PIL path (ImageEnhance / Image.convert: what the reference runs, since its
-    mapper feeds PIL images) -- both bit for bit."""
-    if arithmetic not in ("tensor", "pil"):
-        raise ValueError("arithmetic must be 'tensor' or 'pil'")
-    pil = arithmetic == "pil"
+    order with their ``factors`` (Python floats); an empty order = jitter not applied.  Follows torchvision's PIL path
+    (ImageEnhance / Image.convert: what the reference runs, since its mapper feeds PIL images) in Pillow's arithmetic, bit for bit."""
     x, dev = _u8_batch(images)
     N, _, H, W = x.shape
     if len(params) != N:
@@ -837,11 +822,11 @@ def color_jitter(images: Tensor, params: Sequence[dict], arithmetic: str = "tens
             raise ValueError("order / factors: up to four ops from {0, 1, 2, 3} with one factor each")
         arr[n].n_ops = len(order)
         for k, (o, f) in enumerate(zip(order, fac)):
-            arr[n].op[k], arr[n].factor[k], arr[n].one_minus[k] = int(o), float(f), 1.0 - float(f)
-            if pil and int(o) == 3:
+            arr[n].op[k], arr[n].factor[k] = int(o), float(f)
+            if int(o) == 3:
                 if not -0.5 <= float(f) <= 0.5:
                     raise ValueError("hue factor must lie in [-0.5, 0.5]")
-                arr[n].one_minus[k] = float(int(float(f) * 255) & 0xFF)   # np.int32(hue * 255).astype(np.uint8) of torchvision's PIL path
+                arr[n].hue_shift[k] = int(float(f) * 255) & 0xFF   # np.int32(hue * 255).astype(np.uint8) of torchvision's PIL path
         arr[n].grayscale = int(bool(p.get("grayscale", False)))
     out = torch.empty_like(x)
     if N == 0:
@@ -849,43 +834,8 @@ def color_jitter(images: Tensor, params: Sequence[dict], arithmetic: str = "tens
     with torch.cuda.device(dev), _timed("color_jitter"):
         rec = _struct_array_to_device(arr, dev)
         ws = _workspace(dev, "jitter", 8 * N)
-        fn = _lib.lib().sfod_color_jitter_pil if pil else _lib.lib().sfod_color_jitter
-        check(fn(x.data_ptr(), N, H, W, rec.data_ptr(), ws.data_ptr(), ws.numel(), out.data_ptr(), _stream(dev)), "sfod_color_jitter")
-    return out
-
-
-def gaussian_kernel1d(kernel_size: int, sigma: float) -> Tensor:
-    """torchvision.transforms._functional_tensor._get_gaussian_kernel1d (float32, CPU)."""
-    ksize_half = (kernel_size - 1) * 0.5
-    x = torch.linspace(-ksize_half, ksize_half, steps=kernel_size)
-    pdf = torch.exp(-0.5 * (x / sigma).pow(2))
-    return pdf / pdf.sum()
-
-
-def gaussian_blur(images: Tensor, sigmas: Sequence[Optional[float]], kernel_sizes: Optional[Sequence[int]] = None) -> Tensor:
-    """Separable Gaussian blur of a uint8 batch; ``sigmas[n] is None`` leaves image n untouched.  The kernel size defaults to
-    ``2 * ceil(3 sigma) + 1`` (support +-3 sigma); taps are torchvision's ``_get_gaussian_kernel1d``; reflect padding."""
-    x, dev = _u8_batch(images)
-    N, _, H, W = x.shape
-    if len(sigmas) != N:
-        raise ValueError("one sigma (or None) per image")
-    taps = torch.zeros((max(N, 1), 31), dtype=torch.float32)
-    radius = [0] * N
-    for n, sg in enumerate(sigmas):
-        if sg is None:
-            continue
-        ks = int(kernel_sizes[n]) if kernel_sizes is not None else 2 * max(1, math.ceil(3.0 * float(sg))) + 1
-        if ks % 2 == 0 or ks < 3 or ks > 31:
-            raise ValueError("kernel size must be odd, 3..31")
-        radius[n] = (ks - 1) // 2
-        taps[n, :ks] = gaussian_kernel1d(ks, float(sg))
-    out = torch.empty_like(x)
-    if N == 0:
-        return out
-    with torch.cuda.device(dev), _timed("gaussian_blur"):
-        taps_dev, radius_dev = taps.to(dev), _small_i32(dev, radius)      # named: both must outlive the launch call
-        check(_lib.lib().sfod_gaussian_blur(x.data_ptr(), N, H, W, taps_dev.data_ptr(), radius_dev.data_ptr(), max(radius),
-                                            out.data_ptr(), _stream(dev)), "sfod_gaussian_blur")
+        check(_lib.lib().sfod_color_jitter_pil(x.data_ptr(), N, H, W, rec.data_ptr(), ws.data_ptr(), ws.numel(), out.data_ptr(),
+                                               _stream(dev)), "sfod_color_jitter_pil")
     return out
 
 

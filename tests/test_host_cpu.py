@@ -39,10 +39,10 @@ def test_library_exports_every_declared_symbol():
     assert {e for e in exported if e.startswith("sfod_")} == declared
 
 
-def test_host_only_entry_points_abi_v2():
+def test_host_only_entry_points_abi_v3():
     L = _lib.lib()
     launches = L.sfod_debug_launch_count()                      # non-zero when GPU tests ran earlier in this process
-    assert L.sfod_abi_version() == 2
+    assert L.sfod_abi_version() == 3
     # the ctypes mirrors of the parameter structs have the C layout (sizeof as compiled into the library)
     for which, mirror in enumerate((_lib.EmaTensor, _lib.RpnParams, _lib.FrcnnParams, _lib.P2PComm, _lib.JitterParams, _lib.EraseParams)):
         assert L.sfod_abi_sizeof(which) == C.sizeof(mirror), (which, mirror.__name__, L.sfod_abi_sizeof(which), C.sizeof(mirror))
@@ -85,11 +85,11 @@ def test_host_only_entry_points_abi_v2():
     assert L.sfod_debug_launch_count() == launches              # nothing was launched by any of the above
 
 
-def test_binding_refuses_a_library_of_another_abi(monkeypatch):
+def test_binding_refuses_a_library_of_another_abi_v3(monkeypatch):
     """A library built from another revision of the header would take the binding's argument lists unchecked."""
     monkeypatch.setattr(_lib, "_lib", None)
     monkeypatch.setattr(_lib, "ABI_VERSION", 1)
-    with pytest.raises(_lib.SfodLibraryError, match="ABI version 2, this binding expects 1"):
+    with pytest.raises(_lib.SfodLibraryError, match="ABI version 3, this binding expects 1"):
         _lib.lib()
     monkeypatch.undo()
 
