@@ -431,6 +431,19 @@ typedef struct sfod_resize_image {
 int sfod_resize_pil(const sfod_resize_image *records_dev, int N, const int32_t *coeffs_dev, uint8_t *out, int max_out_h,
                     int max_out_w, int max_ksize, sfod_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------------------------------------
+ * Fully connected layer of the box head in fp32 on the tensor cores: y = act(x W^T + b) with x (M, K), W (N, K) and y (M, N)
+ * row-major fp32 (nn.Linear's layout), b (N) or NULL, act 0 = none, 1 = ReLU (NaN propagates as in torch.relu).
+ * 3xTF32 arithmetic: every operand is split into hi = tf32(v) and lo = tf32(v - hi), and x W^T is accumulated as
+ * lo*hi + hi*lo + hi*hi in fp32, which keeps fp32-level accuracy (the dropped lo*lo term is <= 2^-22 relative per product).
+ * The workspace holds the hi and lo planes of W and of x, rebuilt on every call (W may change in place between calls).
+ * SFOD_ERR_INVALID_ARG for null x / w / y, M < 0, non-positive K or N, or another act; SFOD_ERR_UNSUPPORTED for K % 4 != 0,
+ * N % 16 != 0 or M beyond 65535 * 128; SFOD_ERR_ALIGNMENT unless x, w, y and the workspace are 16-byte aligned.  All
+ * checks happen before any launch.  M == 0 launches nothing. */
+size_t sfod_linear_3xtf32_workspace_bytes(int64_t M, int N, int K);
+int sfod_linear_3xtf32(const float *x, int64_t M, int K, const float *w, int N, const float *bias, int act, float *y,
+                       void *workspace, size_t workspace_bytes, sfod_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

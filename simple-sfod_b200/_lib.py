@@ -104,6 +104,8 @@ SIGNATURES = {
     "sfod_gaussian_blur_pil": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "sfod_random_erase": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_uint64, c_ptr]),
     "sfod_resize_pil": (C.c_int, [c_ptr, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
+    "sfod_linear_3xtf32_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int]),
+    "sfod_linear_3xtf32": (C.c_int, [c_ptr, C.c_int64, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "sfod_subsample_labels": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_uint64, c_ptr, c_ptr, c_ptr]),
     "sfod_bn_stats_bytes": (C.c_size_t, [C.c_int]),
     "sfod_bn_partial_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, C.POINTER(P2PComm), c_ptr]),

@@ -6,7 +6,9 @@ share one body: ROIPooler -> box head -> predictor, then either ``box_predictor.
 path: pooling, decode, per-class NMS, top-k all run in libsfod_b200) or the training losses.  Proposal labelling /
 sampling and the losses (the student's training step, SURVEY.md 8f rank 1) are restated from detectron2 0.6 and the
 reference in plain torch; in that mode the library contributes ROIAlign forward AND backward (autograd) and the decode
-kernels.  The box-head FCs stay on cuBLAS (dense GEMMs are library work per BASELINE.json north_star).
+kernels.  Without autograd and in strict fp32 (``matmul.allow_tf32`` off) the box-head FCs run on the library's 3xTF32
+tensor-core kernel (``ops.linear_3xtf32``: fp32-level accuracy, see ``FastRCNNConvFCHead.forward``); the student's training
+step and TF32 math keep them on cuBLAS.
 """
 from __future__ import annotations
 
@@ -61,6 +63,28 @@ class FastRCNNConvFCHead(nn.Sequential):
             self.add_module("fc_relu{}".format(k + 1), nn.ReLU())
             self.fcs.append(fc)
             self._output_size = fc_dim
+
+    def forward(self, x: Tensor) -> Tensor:
+        """Without autograd, on CUDA fp32 input and with ``matmul.allow_tf32`` off (strict fp32), every FC + ReLU runs as one
+        ``ops.linear_3xtf32`` call (tensor cores, fp32-level accuracy).  Otherwise -- the student's training step, TF32 math,
+        CPU -- the layers run as the ``nn.Sequential`` they are."""
+        if not self._native_fcs(x):
+            return super().forward(x)
+        from .. import ops
+        for k, conv in enumerate(self.conv_norm_relus):
+            x = getattr(self, "conv_relu{}".format(k + 1))(conv(x))
+        x = torch.flatten(x, 1)
+        for fc in self.fcs:   # every fc is followed by its ReLU
+            x = ops.linear_3xtf32(x, fc.weight, fc.bias, relu=True)
+        return x
+
+    def _native_fcs(self, x: Tensor) -> bool:
+        if not self.fcs or not x.is_cuda or x.dtype != torch.float32 or torch.backends.cuda.matmul.allow_tf32:
+            return False
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            return False
+        from .. import ops
+        return all(ops.linear_3xtf32_supported(fc.in_features, fc.out_features) for fc in self.fcs)
 
     @property
     def output_shape(self) -> ShapeSpec:

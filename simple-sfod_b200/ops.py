@@ -630,6 +630,32 @@ def frcnn_postprocess(cls_logits: Tensor, deltas: Tensor, proposals: Tensor, row
                 pseudo_count=pseudo_count, probs=probs, decoded=boxes)
 
 
+# ----------------------------------------------------------------------------------------------- box-head FC
+def linear_3xtf32_supported(in_features: int, out_features: int) -> bool:
+    """Shapes ``linear_3xtf32`` covers (TMA row strides are 16-byte multiples; the epilogue stores groups of 16 columns)."""
+    return in_features % 4 == 0 and out_features % 16 == 0
+
+
+def linear_3xtf32(x: Tensor, weight: Tensor, bias: Optional[Tensor] = None, relu: bool = False) -> Tensor:
+    """``F.linear(x, weight, bias)`` (then ``torch.relu`` when ``relu``) in fp32 on the tensor cores with 3xTF32 arithmetic:
+    fp32-level accuracy whatever ``torch.backends.cuda.matmul.allow_tf32`` says.  x (M, K), weight (N, K); no autograd."""
+    dev = _require_cuda(x, weight, bias)
+    x, w = _f32c(x), _f32c(weight)
+    b = _f32c(bias) if bias is not None else None
+    M, K = x.shape
+    N = w.shape[0]
+    if w.shape[1] != K or (b is not None and b.shape != (N,)):
+        raise ValueError(f"linear_3xtf32: x {tuple(x.shape)}, weight {tuple(w.shape)}, bias {None if b is None else tuple(b.shape)}")
+    y = torch.empty((M, N), dtype=torch.float32, device=dev)
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, "linear_3xtf32", L.sfod_linear_3xtf32_workspace_bytes(M, N, K))
+        with _timed("box_head_fc"):
+            check(L.sfod_linear_3xtf32(x.data_ptr(), M, K, w.data_ptr(), N, b.data_ptr() if b is not None else None, int(bool(relu)),
+                                       y.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)), "sfod_linear_3xtf32")
+    return y
+
+
 # ----------------------------------------------------------------------------------------------- EMA
 class EmaPlan:
     """One-launch mean-teacher EMA over a fixed set of (student, teacher) tensor pairs.
