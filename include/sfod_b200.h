@@ -50,7 +50,8 @@ enum sfod_dtype { SFOD_F32 = 0, SFOD_I64 = 1, SFOD_U8 = 2 };
  * a binding refuses a library of another version. */
 int sfod_abi_version(void);
 /* sizeof() of the parameter structs as this library was compiled (which: 0 sfod_ema_tensor, 1 sfod_rpn_params,
- * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params, 6 sfod_resize_image; 0 for anything else) -- lets a foreign
+ * 2 sfod_frcnn_params, 3 sfod_p2p_comm, 4 sfod_jitter_params, 5 sfod_erase_params, 6 sfod_resize_image, 7 sfod_coco_eval_params;
+ * 0 for anything else) -- lets a foreign
  * binding (ctypes / cffi struct mirrors) check its layout against the C one before the first call. */
 size_t sfod_abi_sizeof(int which);
 const char *sfod_status_string(int status);
@@ -443,6 +444,47 @@ int sfod_resize_pil(const sfod_resize_image *records_dev, int N, const int32_t *
 size_t sfod_linear_3xtf32_workspace_bytes(int64_t M, int N, int K);
 int sfod_linear_3xtf32(const float *x, int64_t M, int K, const float *w, int N, const float *bias, int act, float *y,
                        void *workspace, size_t workspace_bytes, sfod_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------------------------------
+ * COCO box AP (SURVEY.md 8f row f-5): pycocotools' COCOeval(iouType="bbox").evaluate() + accumulate(), bit-equal, as the
+ * reference reaches it through detectron2's COCOEvaluator (reference daod/evaluation/; test_refinement at
+ * daod/engine/trainers/base.py:300, the --eval-only runs of train_net*.py, EvalHook).  summarize() stays with the caller.
+ * Images are the I ground-truth images in ascending image-id order; categories the K ground-truth categories in ascending id
+ * order (an index outside [0, K) is never evaluated, as a result of another category id).
+ * Ground truth (n_gt = gt_offsets[I] entries, device arrays, sorted by image): the gt of image i are rows
+ *   [gt_offsets[i], gt_offsets[i+1]) in annotation order; gt_offsets is HOST memory (I + 1 entries, gt_offsets[0] = 0).
+ *   gt_boxes (n_gt, 4) fp64 XYWH, gt_area fp64 (the annotation's "area", not w * h), gt_iscrowd uint8 (!= 0: crowd),
+ *   gt_ids int64 (the annotation id: a match to id 0 counts as a false positive, as in COCOeval), gt_categories int64.
+ * Detections (device arrays, one padded row of P = dt_stride slots per image, in the order of the caller's result list):
+ *   dt_boxes (I, P, 4) fp32 XYWH (16-byte aligned), dt_scores (I, P) fp32, dt_classes (I, P) int64, dt_counts (I) int32 valid
+ *   slots per row -- device-side, so a detector's padded output is evaluated without reading its counts on the host.
+ * Outputs (device fp64, COCOeval's layouts and -1 conventions): precision and scores (T, R, K, A, M), recall (T, K, A, M).
+ * Thresholds and ranges are taken as given (the caller computes iouThrs / recThrs with numpy's linspace, as Params does).
+ * SFOD_ERR_INVALID_ARG for a null pointer, non-positive sizes, a maxDets entry < 1, gt_offsets[0] != 0 or decreasing gt
+ * offsets (gt not sorted by image); SFOD_ERR_UNSUPPORTED for K > SFOD_COCO_MAX_CATEGORIES, P > 1024, more than 1024 gt in one
+ * image, a maxDets entry > 128, more thresholds / ranges than the arrays below hold, or I * P >= 2^24; SFOD_ERR_ALIGNMENT
+ * for dt_boxes.  All checks happen before any launch. */
+#define SFOD_COCO_MAX_CATEGORIES 254
+#define SFOD_COCO_MAX_IOU_THRS 16
+#define SFOD_COCO_MAX_REC_THRS 128
+#define SFOD_COCO_MAX_AREA_RNGS 4
+#define SFOD_COCO_MAX_MAX_DETS 4
+typedef struct sfod_coco_eval_params {
+  int32_t n_images;                               /* I */
+  int32_t n_categories;                           /* K */
+  int32_t dt_stride;                              /* P: detection slots per image row */
+  int32_t n_iou_thrs, n_rec_thrs, n_area_rngs, n_max_dets;   /* T, R, A, M */
+  int32_t max_dets[SFOD_COCO_MAX_MAX_DETS];       /* maxDets; the last one truncates every (image, category) */
+  int32_t reserved;
+  double iou_thrs[SFOD_COCO_MAX_IOU_THRS];
+  double rec_thrs[SFOD_COCO_MAX_REC_THRS];
+  double area_rng[SFOD_COCO_MAX_AREA_RNGS][2];    /* inclusive [lo, hi] on the area */
+} sfod_coco_eval_params;
+size_t sfod_coco_eval_workspace_bytes(const sfod_coco_eval_params *p);
+int sfod_coco_eval(const sfod_coco_eval_params *p, const int64_t *gt_offsets, const double *gt_boxes, const double *gt_area,
+                   const uint8_t *gt_iscrowd, const int64_t *gt_ids, const int64_t *gt_categories, const float *dt_boxes,
+                   const float *dt_scores, const int64_t *dt_classes, const int32_t *dt_counts, double *precision, double *scores,
+                   double *recall, void *workspace, size_t workspace_bytes, sfod_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -53,6 +53,16 @@ class FrcnnParams(C.Structure):
                 ("coord_trick_max_n", C.c_int64), ("rows_stride", C.c_int)]
 
 
+COCO_MAX_CATEGORIES, COCO_MAX_IOU_THRS, COCO_MAX_REC_THRS, COCO_MAX_AREA_RNGS, COCO_MAX_MAX_DETS = 254, 16, 128, 4, 4
+
+
+class CocoEvalParams(C.Structure):
+    _fields_ = [("n_images", C.c_int32), ("n_categories", C.c_int32), ("dt_stride", C.c_int32), ("n_iou_thrs", C.c_int32),
+                ("n_rec_thrs", C.c_int32), ("n_area_rngs", C.c_int32), ("n_max_dets", C.c_int32),
+                ("max_dets", C.c_int32 * COCO_MAX_MAX_DETS), ("reserved", C.c_int32), ("iou_thrs", C.c_double * COCO_MAX_IOU_THRS),
+                ("rec_thrs", C.c_double * COCO_MAX_REC_THRS), ("area_rng", (C.c_double * 2) * COCO_MAX_AREA_RNGS)]
+
+
 P2P_MAX_RANKS = 8
 P2P_HANDLE_BYTES = 64
 
@@ -63,7 +73,7 @@ class P2PComm(C.Structure):
 
 # sfod_abi_version() of the library this binding is written for, and the struct mirrors in the order of sfod_abi_sizeof(which)
 ABI_VERSION = 3
-ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams, ResizeImage)
+ABI_STRUCTS = (EmaTensor, RpnParams, FrcnnParams, P2PComm, JitterParams, EraseParams, ResizeImage, CocoEvalParams)
 
 
 # name -> (restype, argtypes); every symbol include/sfod_b200.h declares
@@ -106,6 +116,8 @@ SIGNATURES = {
     "sfod_resize_pil": (C.c_int, [c_ptr, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
     "sfod_linear_3xtf32_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int]),
     "sfod_linear_3xtf32": (C.c_int, [c_ptr, C.c_int64, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int, c_ptr, c_ptr, C.c_size_t, c_ptr]),
+    "sfod_coco_eval_workspace_bytes": (C.c_size_t, [C.POINTER(CocoEvalParams)]),
+    "sfod_coco_eval": (C.c_int, [C.POINTER(CocoEvalParams)] + [c_ptr] * 14 + [C.c_size_t, c_ptr]),
     "sfod_subsample_labels": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_uint64, c_ptr, c_ptr, c_ptr]),
     "sfod_bn_stats_bytes": (C.c_size_t, [C.c_int]),
     "sfod_bn_partial_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int64, c_ptr, C.POINTER(P2PComm), c_ptr]),

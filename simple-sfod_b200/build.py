@@ -13,7 +13,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsfod_b200.so")
-SOURCES = ["ema.cu", "roi.cu", "detect.cu", "bn.cu", "image.cu", "augment.cu", "resize.cu", "linear.cu"]
+SOURCES = ["ema.cu", "roi.cu", "detect.cu", "bn.cu", "image.cu", "augment.cu", "resize.cu", "linear.cu", "evaluate.cu"]
 # -fmad=false: parity-critical arithmetic must not be contracted into FMAs; kernels that want FMAs call fmaf().
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "--threads", "2"]

@@ -426,6 +426,7 @@ SFOD_API size_t sfod_abi_sizeof(int which) {
     case 4: return sizeof(sfod_jitter_params);
     case 5: return sizeof(sfod_erase_params);
     case 6: return sizeof(sfod_resize_image);
+    case 7: return sizeof(sfod_coco_eval_params);
     default: return 0;
   }
 }

@@ -15,6 +15,7 @@
 //   j >= keys/CTA : distributed-shared-memory exchange between the CTAs of a thread-block cluster (a 16 384-key tile is
 //                   spread over 8 CTAs = 8 SMs x 4 warps instead of 32 warps queueing on one SM),
 //   j >= tile     : global-memory exchange kernel (only when P > 16384, e.g. 34 200 R101 anchors).
+// The kernels have internal linkage: every translation unit that sorts (detect.cu, evaluate.cu) holds its own copy.
 #pragma once
 #include "common.cuh"
 
@@ -142,7 +143,7 @@ __device__ __forceinline__ void block_bitonic(unsigned long long (&a)[kE], unsig
 
 // Tile kernel: grid (cl * P / tile, S) launched as clusters of cl CTAs along x; block tile/cl/16 threads; dynamic smem
 // tile/cl*8 bytes.
-__global__ void __launch_bounds__(kClusterMinKeys / kE) bitonic_tile_kernel(unsigned long long *keys, int P, int tile, int cl, int k_lo, int k_hi) {
+static __global__ void __launch_bounds__(kClusterMinKeys / kE) bitonic_tile_kernel(unsigned long long *keys, int P, int tile, int cl, int k_lo, int k_hi) {
   extern __shared__ unsigned long long sort_smem[];
   const int ctile = tile / cl, rank = (int)(blockIdx.x % (unsigned)cl);
   unsigned long long *seg = keys + (size_t)blockIdx.y * P + (size_t)blockIdx.x * ctile;
@@ -159,7 +160,7 @@ __global__ void __launch_bounds__(kClusterMinKeys / kE) bitonic_tile_kernel(unsi
 }
 
 // Global exchange for one stage (k, j) with j >= tile: grid (P/2/256, S), block 256.
-__global__ void __launch_bounds__(256) bitonic_global_kernel(unsigned long long *keys, int P, long long k, long long j) {
+static __global__ void __launch_bounds__(256) bitonic_global_kernel(unsigned long long *keys, int P, long long k, long long j) {
   unsigned long long *seg = keys + (size_t)blockIdx.y * P;
   const long long tt = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (tt >= P / 2) return;

@@ -10,3 +10,4 @@ from .export import (batch_to_coco_json, detector_postprocess, instances_to_coco
 from .hooks import HookBase, TeacherEMAHook, TrainerBase  # noqa: F401
 from .augment import draw_params as draw_strong_augmentation_params, strong_augment  # noqa: F401
 from .augment import apply_weak_to_boxes, draw_weak_params, weak_augment  # noqa: F401
+from .evaluation import COCOBoxEvaluator, inference_on_dataset  # noqa: F401

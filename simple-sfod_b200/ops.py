@@ -1076,3 +1076,80 @@ def resize_pil(images: Union[Tensor, Sequence[Tensor]], sizes: Sequence[Tuple[in
     if all(s == sz[0] for s in sz):
         return out.view(N, 3, sz[0][0], sz[0][1])
     return [out[o:o + 3 * h * w].view(3, h, w) for o, (h, w) in zip(plan.offsets, sz)]
+
+
+# ----------------------------------------------------------------------------------------------- COCO box AP
+def coco_eval_out_numel(T: int, R: int, K: int, A: int, M: int) -> int:
+    """Elements of the packed fp64 result of ``coco_box_eval``: precision and scores (T, R, K, A, M), then recall (T, K, A, M)."""
+    return 2 * T * R * K * A * M + T * K * A * M
+
+
+def coco_box_eval(gt_offsets: Sequence[int], gt_boxes: Tensor, gt_area: Tensor, gt_iscrowd: Tensor, gt_ids: Tensor, gt_categories: Tensor,
+                  dt_boxes: Tensor, dt_scores: Tensor, dt_classes: Tensor, dt_counts: Tensor, num_categories: int,
+                  iou_thrs: Sequence[float], rec_thrs: Sequence[float], area_rngs: Sequence[Sequence[float]], max_dets: Sequence[int],
+                  out: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
+    """pycocotools ``COCOeval(iouType="bbox")``: ``evaluate()`` + ``accumulate()`` on the device, bit-equal (include/sfod_b200.h,
+    ``sfod_coco_eval``).  Images are the ground truth's images in ascending id order, categories its categories in ascending
+    id order (index 0..K-1).
+
+    ``gt_offsets`` (host, I + 1 ints): the gt of image i are rows [gt_offsets[i], gt_offsets[i+1]) of ``gt_boxes`` (n_gt, 4)
+    fp64 XYWH, ``gt_area`` fp64 (the annotations' area), ``gt_iscrowd``, ``gt_ids`` and ``gt_categories`` int64, in annotation
+    order.  Detections: one padded row per image, ``dt_boxes`` (I, P, 4) fp32 XYWH, ``dt_scores`` (I, P), ``dt_classes``
+    (I, P) int64 and the device-side valid counts ``dt_counts`` (I).  ``out``: optional fp64 buffer of at least
+    ``coco_eval_out_numel`` elements.  Returns (precision, recall, scores) as views into it, with COCOeval's -1 where a cell is
+    undefined.  No host synchronisation."""
+    dev = _require_cuda(gt_boxes, gt_area, gt_iscrowd, gt_ids, gt_categories, dt_boxes, dt_scores, dt_classes, dt_counts, out)
+    offs = [int(v) for v in gt_offsets]
+    I = len(offs) - 1
+    if I < 0 or offs[0] != 0 or any(b < a for a, b in zip(offs, offs[1:])):
+        raise ValueError("coco_box_eval: gt_offsets must start at 0 and be non-decreasing (ground truth sorted by image)")
+    n_gt = offs[-1]
+    if max((b - a for a, b in zip(offs, offs[1:])), default=0) > 1024:
+        raise ValueError("coco_box_eval: more than 1024 ground-truth boxes in one image")
+    if tuple(gt_boxes.shape) != (n_gt, 4) or any(t.shape != (n_gt,) for t in (gt_area, gt_iscrowd, gt_ids, gt_categories)):
+        raise ValueError(f"coco_box_eval: ground truth of {n_gt} boxes expected, got boxes {tuple(gt_boxes.shape)}")
+    if dt_boxes.dim() != 3 or dt_boxes.shape[0] != I or dt_boxes.shape[2] != 4:
+        raise ValueError(f"coco_box_eval: dt_boxes must be ({I}, P, 4), got {tuple(dt_boxes.shape)}")
+    P = dt_boxes.shape[1]
+    if dt_scores.shape != (I, P) or dt_classes.shape != (I, P) or dt_counts.shape != (I,):
+        raise ValueError("coco_box_eval: dt_scores / dt_classes must be (I, P) and dt_counts (I,)")
+    if not 1 <= P <= 1024 or I * P >= 1 << 24:
+        raise ValueError(f"coco_box_eval: {P} detection slots per image (1..1024, images x slots < 2^24)")
+    K, T, R, A, M = int(num_categories), len(iou_thrs), len(rec_thrs), len(area_rngs), len(max_dets)
+    if not (1 <= K <= _lib.COCO_MAX_CATEGORIES and 1 <= T <= _lib.COCO_MAX_IOU_THRS and 1 <= R <= _lib.COCO_MAX_REC_THRS
+            and 1 <= A <= _lib.COCO_MAX_AREA_RNGS and 1 <= M <= _lib.COCO_MAX_MAX_DETS):
+        raise ValueError(f"coco_box_eval: unsupported sizes K={K} T={T} R={R} A={A} M={M}")
+    if any(not 1 <= int(m) <= 128 for m in max_dets):
+        raise ValueError(f"coco_box_eval: maxDets must lie in 1..128, got {list(max_dets)}")
+    if any(t.dtype != d for t, d in ((gt_boxes, torch.float64), (gt_area, torch.float64), (gt_ids, torch.int64), (gt_categories, torch.int64),
+                                     (dt_boxes, torch.float32), (dt_scores, torch.float32), (dt_classes, torch.int64), (dt_counts, torch.int32))):
+        raise ValueError("coco_box_eval: gt boxes / area fp64, ids / categories / dt classes int64, dt boxes / scores fp32, counts int32")
+    need = coco_eval_out_numel(T, R, K, A, M)
+    if out is None:
+        out = torch.empty(need, dtype=torch.float64, device=dev)
+    elif out.dtype != torch.float64 or not out.is_contiguous() or out.numel() < need:
+        raise ValueError(f"coco_box_eval: out must be a contiguous fp64 tensor of >= {need} elements")
+    p = _lib.CocoEvalParams()
+    p.n_images, p.n_categories, p.dt_stride = I, K, P
+    p.n_iou_thrs, p.n_rec_thrs, p.n_area_rngs, p.n_max_dets = T, R, A, M
+    for i, v in enumerate(max_dets):
+        p.max_dets[i] = int(v)
+    for i, v in enumerate(iou_thrs):
+        p.iou_thrs[i] = float(v)
+    for i, v in enumerate(rec_thrs):
+        p.rec_thrs[i] = float(v)
+    for i, (lo, hi) in enumerate(area_rngs):
+        p.area_rng[i][0], p.area_rng[i][1] = float(lo), float(hi)
+    host_offs = (C.c_int64 * (I + 1))(*offs)
+    gt = [t.contiguous() for t in (gt_boxes, gt_area, gt_iscrowd.to(torch.uint8), gt_ids, gt_categories)]
+    dt = [t.contiguous() for t in (dt_boxes, dt_scores, dt_classes, dt_counts)]
+    n1 = T * R * K * A * M
+    precision, scores, recall = out[:n1], out[n1:2 * n1], out[2 * n1:need]
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, "coco_eval", L.sfod_coco_eval_workspace_bytes(C.byref(p)))
+        with _timed("coco_eval"):
+            check(L.sfod_coco_eval(C.byref(p), host_offs, *[_ptr(t) if t.numel() else None for t in gt], *[_ptr(t) if t.numel() else None for t in dt],
+                                   precision.data_ptr(), scores.data_ptr(), recall.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)),
+                  "sfod_coco_eval")
+    return precision.view(T, R, K, A, M), recall.view(T, K, A, M), scores.view(T, R, K, A, M)
