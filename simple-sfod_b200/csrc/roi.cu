@@ -1128,6 +1128,12 @@ SFOD_API size_t sfod_roi_align_fwd_workspace_bytes(int N, int C, int H, int W, i
   size_t bytes = need ? sfod_align_up((size_t)N * C * H * W * sizeof(float), 256) : 0;
   if (!exact) bytes += 256 + sfod_align_up((size_t)(R > 0 ? R : 0) * sep_rec_floats(H) * sizeof(float), 256) +
                        sfod_align_up((size_t)(R > 0 ? R : 0) * kCostClasses * sizeof(int), 256);
+  // a channels-last call falls back to the exact kernel (which reads an NCHW copy) when the separable path does not support
+  // the shape -- C % 4, the map size, or an output other than 7 x 7, which this query is not told
+  if (!exact && layout == SFOD_NHWC) {
+    const size_t nchw = sfod_align_up((size_t)N * C * H * W * sizeof(float), 256);
+    if (bytes < nchw) bytes = nchw;
+  }
   return bytes ? bytes : 256;
 }
 

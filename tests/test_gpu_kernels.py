@@ -202,10 +202,10 @@ def test_roi_align_kat_and_api(ops, cuda_device):
 
 @pytest.mark.parametrize("cfg", [synth.V, synth.R101, dict(name="mid-even-W", C=48, H=40, W=50, stride=16)], ids=["V", "R", "mid"])
 def test_roi_align_forward_any_image_order_and_invalid_index(ops, cuda_device, cfg):
-    """The slab-resident forwards (32-channel slab: V; 16-channel slab with two half-warps per ROI: R101-C4 and the 40 x 50 map,
-    whose even row length is padded to an odd stride) serve the ROIs of one image at a time from shared memory: ROIs must be
-    accepted in any image order (detectron2 passes them grouped by image, torchvision's API does not require it), images
-    without ROIs are skipped, and an out-of-range batch index yields zeros (library contract; torchvision reads out of bounds)."""
+    """The slab-resident forward (32-channel slab: V) serves the ROIs of one image at a time from shared memory; R101-C4 and
+    the 40 x 50 map, whose slabs do not fit, run the persistent L2 forward.  ROIs must be accepted in any image order
+    (detectron2 passes them grouped by image, torchvision's API does not require it), images without ROIs are skipped, and an
+    out-of-range batch index yields zeros (library contract; torchvision reads out of bounds)."""
     N, R = (5, 700) if cfg["C"] <= 512 else (3, 260)
     x = synth.features(cfg, N, 51)
     rois = synth.random_rois(N, R, 52)
