@@ -5,15 +5,18 @@ daod/engine/trainers/base.py:300, the --eval-only runs of train_net*.py, EvalHoo
 ``COCOeval.evaluate`` + ``accumulate`` run on the device in one library call (``ops.coco_box_eval``, bit-equal to pycocotools);
 ``summarize`` and detectron2's ``_derive_coco_results`` run here on the host in numpy over the arrays the device returned, so
 their summation order is pycocotools' own.  ``process`` keeps the detections on the device without synchronising; ``evaluate``
-packs them, makes one library call and one device->host copy.
+packs them, makes one library call and one device->host copy.  In a distributed run every rank's detections are gathered
+onto the main rank first, as detectron2's ``COCOEvaluator(distributed=True)`` does.
 """
 from __future__ import annotations
 
 import json
+import os
 from typing import Dict, List, Optional, Sequence, Union
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from .. import ops
 from .export import _xyxy_to_xywh
@@ -25,6 +28,8 @@ MAX_DETS = [1, 10, 100]
 AREA_RNG = [[0 ** 2, 1e5 ** 2], [0 ** 2, 32 ** 2], [32 ** 2, 96 ** 2], [96 ** 2, 1e5 ** 2]]
 AREA_RNG_LBL = ["all", "small", "medium", "large"]
 METRICS = ["AP", "AP50", "AP75", "APs", "APm", "APl"]
+
+_UNKNOWN_IMAGE = "Results do not correspond to current coco set: detections on an image the ground truth does not list"
 
 
 def summarize(precision: np.ndarray, recall: np.ndarray) -> np.ndarray:
@@ -77,9 +82,21 @@ class COCOBoxEvaluator:
     ``class_names`` defaults to the category names in that order.  ``evaluate`` returns detectron2's
     ``{"bbox": {"AP", "AP50", "AP75", "APs", "APm", "APl", "AP-<name>", ...}}`` and leaves COCOeval's arrays and the 12
     summary stats in ``self.eval`` (per-class AP50: ``self.eval["precision"][0, :, :, 0, -1].mean(axis=0)``).  A detection on an
-    image the ground truth does not list makes ``evaluate`` raise, as ``COCO.loadRes`` does."""
+    image the ground truth does not list makes ``evaluate`` raise, as ``COCO.loadRes`` does.
 
-    def __init__(self, coco_gt: Union[dict, str], class_names: Optional[Sequence[str]] = None):
+    ``distributed`` (detectron2's keyword): when ``torch.distributed`` is initialised with more than one rank, ``evaluate``
+    gathers the detections of every rank of the default group onto rank 0, in rank order, and evaluates them there; the other
+    ranks return ``{}`` and leave ``self.eval`` all None.  Every rank must call ``evaluate``, and every rank raises when the
+    evaluation fails.  With ``distributed=False`` each process evaluates what it processed itself.
+
+    ``output_dir``: rank 0 also writes ``output_dir/coco_instances_results.json``, detectron2's COCO result list (the kept
+    detections in processing order and, distributed, rank order; boxes XYWH in the input's frame; dataset category ids), the
+    list ``engine.prediction_to_gt`` turns into pseudo-labels."""
+
+    def __init__(self, coco_gt: Union[dict, str], class_names: Optional[Sequence[str]] = None, *, distributed: bool = True,
+                 output_dir: Optional[str] = None):
+        self._distributed = distributed
+        self._output_dir = output_dir
         if isinstance(coco_gt, (str, bytes)) or hasattr(coco_gt, "__fspath__"):
             with open(coco_gt) as f:
                 coco_gt = json.load(f)
@@ -143,15 +160,18 @@ class COCOBoxEvaluator:
         """-> ``{"bbox": {"AP", "AP50", "AP75", "APs", "APm", "APl", "AP-<name>", ...}}`` (detectron2's result: a nested dict of
         floats, as ``EvalHook`` requires), ``{}`` when nothing was processed.  COCOeval's arrays stay on the evaluator:
         ``self.eval = {"precision": (T, R, K, A, M), "recall": (T, K, A, M), "scores": (T, R, K, A, M), "stats": (12,)}``
-        (numpy; all None when there was not a single detection, as detectron2 then skips COCOeval)."""
+        (numpy; all None when there was not a single detection, as detectron2 then skips COCOeval).  Distributed: the result on
+        rank 0, ``{}`` on the other ranks."""
         self.eval = {"precision": None, "recall": None, "scores": None, "stats": None}
-        if not self._records:
+        gather = self._distributed and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+        records = self._gather_records() if gather else self._records
+        if not records:                                  # other ranks (None), or nothing processed anywhere
             return {}                                    # detectron2: "did not receive valid predictions"
-        dev = self._records[0][1].device
+        dev = records[0][1].device
         if dev.type != "cuda":
             raise RuntimeError("COCOBoxEvaluator evaluates on the GPU (no CPU fallback); got detections on " + str(dev))
         K = len(self.cat_ids)
-        packed = self._pack(dev)
+        packed = self._pack(dev, records)
         T, R, A, M = len(IOU_THRS), len(REC_THRS), len(AREA_RNG), len(MAX_DETS)
         n_out = ops.coco_eval_out_numel(T, R, K, A, M)
         buf = torch.empty(n_out + 2, dtype=torch.float64, device=dev)
@@ -162,7 +182,9 @@ class COCOBoxEvaluator:
                           packed["classes"], packed["counts"], K, IOU_THRS, REC_THRS, AREA_RNG, MAX_DETS, out=buf)
         res = buf.cpu().numpy()                          # the one device->host copy
         if res[n_out + 1] > 0:
-            raise ValueError("Results do not correspond to current coco set: detections on an image the ground truth does not list")
+            raise ValueError(_UNKNOWN_IMAGE)
+        if self._output_dir is not None and (not dist.is_available() or not dist.is_initialized() or dist.get_rank() == 0):
+            self._write_results(records)
         if res[n_out] == 0:                              # detectron2 skips COCOeval without a single detection
             return {"bbox": derive_coco_results(None, None, self.class_names)}
         n1 = T * R * K * A * M
@@ -172,7 +194,74 @@ class COCOBoxEvaluator:
         self.eval = {"precision": precision, "recall": recall, "scores": res[n1:2 * n1].reshape(T, R, K, A, M), "stats": stats}
         return {"bbox": derive_coco_results(stats, precision, self.class_names)}
 
-    def _pack(self, dev: torch.device) -> Dict[str, torch.Tensor]:
+    def _gather_records(self) -> Optional[list]:
+        """Every rank's records, in rank order then processing order, on rank 0 (the list ``itertools.chain(*comm.gather(...))``
+        leaves in detectron2), None on the other ranks.  Every rank enters the same two collectives whatever it holds:
+
+        1. ``all_gather_object`` of the host-known metadata: (image id, width) per record and the device of detections that
+           are not on a GPU.  Every rank then raises the same error for a condition that fails the evaluation;
+        2. ``all_gather`` of one padded fp32 (n_max, 7) tensor per rank: XYWH, score, class index, kept flag per entry
+           (``_entries``, computed on the device: no count is read on the host).
+
+        Every rank holds the whole gathered list afterwards, so a kept detection on an image outside the ground truth, which
+        fails the evaluation on rank 0 (``loadRes``), makes the other ranks raise the same error too."""
+        rank, world = dist.get_rank(), dist.get_world_size()
+        recs = self._records
+        not_gpu = next((str(r[1].device) for r in recs if r[1].device.type != "cuda"), None)
+        meta = [None] * world
+        dist.all_gather_object(meta, ([(r[0], r[1].shape[0]) for r in recs], not_gpu))
+        for r, (_, dev) in enumerate(meta):
+            if dev is not None:
+                raise RuntimeError(f"COCOBoxEvaluator evaluates on the GPU (no CPU fallback); got detections on {dev} on rank {r}")
+        if not any(m for m, _ in meta):
+            return [] if rank == 0 else None
+        self._row_width([x for m, _ in meta for x in m])        # raises on every rank
+        n_max = max(1, max(sum(w for _, w in m) for m, _ in meta))
+        dev = recs[0][1].device if recs else torch.device("cuda", torch.cuda.current_device())
+        mine = _entries(recs, dev)
+        payload = torch.zeros(n_max, 7, dtype=torch.float32, device=dev)
+        payload[:mine.shape[0]] = mine
+        parts = [torch.empty_like(payload) for _ in range(world)]
+        dist.all_gather(parts, payload)
+        gathered = []
+        for (m, _), part in zip(meta, parts):
+            offsets = np.cumsum([0] + [w for _, w in m]).tolist()
+            for (img, w), o in zip(m, offsets):
+                e = part[o:o + w]
+                gathered.append((img, e[:, :4], e[:, 4], e[:, 5].to(torch.int64), w, e[:, 6] > 0))
+        if rank == 0:
+            return gathered
+        unknown = [r[5] for r in gathered if r[0] not in self._img_index]
+        if unknown and bool(torch.cat(unknown).any()):
+            raise ValueError(_UNKNOWN_IMAGE)
+        return None
+
+    def _write_results(self, records) -> None:
+        """``output_dir/coco_instances_results.json``: the kept detections of ``records`` as detectron2's COCOEvaluator writes
+        them, the values ``export.instances_to_coco_json(export.detector_postprocess(...), image_id, id_map)`` gives."""
+        rows = _entries(records, records[0][1].device).cpu()      # the json's one device->host copy
+        image_ids = [r[0] for r in records for _ in range(r[1].shape[0])]
+        kept = (rows[:, 6] > 0).tolist()
+        boxes, scores, classes = rows[:, :4].tolist(), rows[:, 4].tolist(), rows[:, 5].to(torch.int64).tolist()
+        results = [{"image_id": img, "category_id": self.cat_ids[classes[k]], "bbox": boxes[k], "score": scores[k]}
+                   for k, img in enumerate(image_ids) if kept[k]]
+        os.makedirs(self._output_dir, exist_ok=True)
+        with open(os.path.join(self._output_dir, "coco_instances_results.json"), "w") as f:
+            json.dump(results, f)
+
+    def _row_width(self, meta) -> int:
+        """P of ``_pack`` for records given as (image id, width): the sum of the record widths of the widest ground-truth image."""
+        row_width = [0] * max(len(self.img_ids), 1)
+        for img, w in meta:
+            n = self._img_index.get(img, -1)
+            if n >= 0:
+                row_width[n] += w
+        P = max(1, max(row_width))
+        if P > 1024:
+            raise ValueError(f"{P} detections for one image: at most 1024 are supported")
+        return P
+
+    def _pack(self, dev: torch.device, recs) -> Dict[str, torch.Tensor]:
         """The processed detections in the library's layout, built on the device without reading any count on the host.
 
         The library wants one padded row of P slots per ground-truth image (ascending image id) with the image's detections in
@@ -192,17 +281,10 @@ class COCOBoxEvaluator:
         1 0 1 1, exclusive prefix 0 1 1 2, start of image 0 = entry 0 -> slots 0 - 1 2; A1 goes to the spare column; row 0 =
         [A0, B0, B1], count 3.  P is the sum of the record widths of the widest image (known on the host)."""
         I = len(self.img_ids)
-        recs = self._records
         img_of = [self._img_index.get(r[0], -1) for r in recs]
         order = sorted(range(len(recs)), key=lambda r: (img_of[r] < 0, img_of[r]))
         widths = [recs[r][1].shape[0] for r in order]
-        row_width = [0] * max(I, 1)
-        for r, w in zip(order, widths):
-            if img_of[r] >= 0:
-                row_width[img_of[r]] += w
-        P = max(1, max(row_width))
-        if P > 1024:
-            raise ValueError(f"{P} detections for one image: at most 1024 are supported")
+        P = self._row_width([(r[0], r[1].shape[0]) for r in recs])
         # per flat entry (host-known): its record, its index within the record, its image (-1: unknown), the start of its group
         rec_e = np.repeat(np.arange(len(order)), widths)
         idx_e = np.concatenate([np.arange(w) for w in widths])
@@ -235,6 +317,18 @@ class COCOBoxEvaluator:
         out["n_results"] = kept.sum()
         out["n_unknown"] = (kept & ~known).sum()
         return out
+
+
+def _entries(records, dev: torch.device) -> torch.Tensor:
+    """(n, 7) fp32 on ``dev``, one row per entry of ``records`` in order: XYWH, score, class index, kept (1 / 0: inside the
+    record's count and not emptied by the post-processing).  Class indices are < 2^24, so exact in fp32; the class of an
+    entry that is not kept is written as 0."""
+    rows = []
+    for _, boxes, scores, classes, count, keep in records:
+        kept = (torch.arange(boxes.shape[0], device=boxes.device) < count) & keep
+        rows.append(torch.cat([boxes, scores[:, None], torch.where(kept, classes, 0)[:, None].to(torch.float32),
+                               kept[:, None].to(torch.float32)], dim=1))
+    return torch.cat(rows) if rows else torch.zeros((0, 7), dtype=torch.float32, device=dev)
 
 
 def _postprocess_boxes(boxes, image_size, height, width):
